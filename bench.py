@@ -412,7 +412,11 @@ def main():
     ap.add_argument("--batch", type=int, default=512)
     ap.add_argument("--no-driver", action="store_true", help="skip the e2e_driver extra (solvers.coneqp n=4096)")
     ap.add_argument("--no-i8", action="store_true", help="skip the extra leg on the experimental int8-slice SYRK")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the solutions of the last timed step (x and z of both solves, float64) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.m <= 0:
         args.m = 2 * args.n
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
@@ -450,12 +454,16 @@ def main():
     zs = [torch.from_numpy(rng.standard_normal(m)).to(dev) for _ in range(2)]
     xw, zw = torch.empty_like(xs[0]), torch.empty_like(zs[0])
 
-    def step_dev():
+    def step_dev(keep=None):
         kkt.factor_ptr(d=d_d.data_ptr(), di=d_di.data_ptr(), space=_lib.DEVICE)
         for i in range(2):
             xw.copy_(xs[i]); zw.copy_(zs[i])
             torch.cuda.current_stream().synchronize()
             kkt.solve_ptr(xw.data_ptr(), zw.data_ptr(), space=_lib.DEVICE)
+            if keep is not None:
+                # the library solves on its own stream and returns once the solution is in xw / zw
+                keep["x_rhs%d" % i] = xw.clone()
+                keep["z_rhs%d" % i] = zw.clone()
 
     def barrier():
         if world > 1:
@@ -465,12 +473,13 @@ def main():
     for _ in range(args.warmup):
         step_dev()
     syrk_ms, potrf_ms, fac_ms, sol_ms, mma_ms = [], [], [], [], []
+    outputs = {}
     barrier()
     launches0 = cvxopt_b200.launch_count()
     with ClockSampler(local_rank) as clk:
         kkt.timer_start()
-        for _ in range(args.steps):
-            step_dev()
+        for k in range(args.steps):
+            step_dev(outputs if k == args.steps - 1 and args.dump_outputs else None)
             b = kkt.last_breakdown()
             syrk_ms.append(b["syrk_ms"]); potrf_ms.append(b["potrf_ms"])
             if "syrk_mma_ms" in b:
@@ -485,6 +494,11 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = float(t.item()) / args.steps
     value = world * f_it / (ms_step * 1e-3) * 1e-9
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives: the directions x, z of the step's two solves (n + m values each)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, v in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), v.cpu().numpy().astype(np.float64))
 
     # ---------------- end-to-end arm (host buffers through the plugin API) ----------------
     def pinned(a):

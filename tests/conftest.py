@@ -23,10 +23,20 @@ def _ref_available():
 def ref():
     """The unmodified reference (cvxopt) built into oracle/_ref by oracle/build_ref.sh."""
     if not _ref_available():
-        pytest.skip("oracle/_ref not built (run oracle/build_ref.sh where /root/reference exists)")
+        pytest.skip("oracle/_ref not built (oracle/build_ref.sh builds it from the reference's sources)")
     if REF_DIR not in sys.path:
         sys.path.insert(0, REF_DIR)
     import cvxopt
     from cvxopt import solvers
     solvers.options["show_progress"] = False
     return cvxopt
+
+
+@pytest.fixture
+def ref_golden(request):
+    """ref_golden(label, compute) -> the reference's stored result (tests/reference_results.py)"""
+    import reference_results
+
+    def get(label, compute):
+        return reference_results.result(request.node, label, compute)
+    return get

@@ -1,6 +1,6 @@
-"""Batch / device-resident IPM (BASELINE config 4) vs the reference: a Python loop over
-solvers.qp (oracle/_ref) on the same problems — same status, same iteration count per problem,
-objectives to rtol 1e-8, x to 1e-6."""
+"""Batch / device-resident IPM (BASELINE config 4) vs the reference: a Python loop over solvers.qp on the same
+problems (its stored results, tests/reference_results.py) — same status, same iteration count per problem, objectives
+to rtol 1e-8, x to 1e-6."""
 import numpy as np
 import pytest
 
@@ -17,20 +17,23 @@ def make_batch(B, n, m, seed0=0):
     return np.stack(Ps), np.stack(qs), np.stack(Gs), np.stack(hs)
 
 
-def ref_loop(ref, P, q, G, h):
+def ref_loop(P, q, G, h):
     from cvxopt import matrix, solvers
-    out = []
+    out = {}
     for k in range(P.shape[0]):
-        out.append(solvers.qp(matrix(P[k]), matrix(q[k]), matrix(G[k]), matrix(h[k]), kktsolver="chol"))
+        sol = solvers.qp(matrix(P[k]), matrix(q[k]), matrix(G[k]), matrix(h[k]), kktsolver="chol")
+        out.update({"%d.%s" % (k, key): sol[key] for key in ("status", "iterations", "primal objective",
+                                                               "dual objective", "x", "s", "z")})
     return out
 
 
 @pytest.mark.parametrize("B,n,m", [(5, 30, 70), (3, 150, 321), (2, 257, 300), (1, 300, 640)])
-def test_batch_matches_reference_loop(ref, B, n, m):
+def test_batch_matches_reference_loop(ref_golden, B, n, m):
     import cvxopt_b200
     P, q, G, h = make_batch(B, n, m, seed0=10 * B)
+    ref = ref_golden("qp_loop", lambda: ref_loop(P, q, G, h))
+    want = [{key.split(".", 1)[1]: v for key, v in ref.items() if key.split(".", 1)[0] == str(k)} for k in range(B)]
     got = cvxopt_b200.qp_batch(P, q, G, h)
-    want = ref_loop(ref, P, q, G, h)
     for k in range(B):
         assert got["status"][k] == want[k]["status"] == "optimal"
         assert got["iterations"][k] == want[k]["iterations"], (k, got["iterations"], want[k]["iterations"])

@@ -1,6 +1,7 @@
 """cvxopt_b200.conelp — the device-resident restatement of coneprog.conelp (every vector in HBM, only scalars cross
-PCIe) against the reference's own solvers.conelp(..., kktsolver='chol') on the same problems: same status, same
-iteration count, objectives to rtol 1e-8; and BASELINE configs 3 and 5 against the reference's committed runs."""
+PCIe) against the reference's own solvers.conelp(..., kktsolver='chol') on the same problems (its stored results,
+tests/reference_results.py): same status, same iteration count, objectives to rtol 1e-8; and BASELINE configs 3 and 5
+against the reference's committed runs."""
 import json
 import os
 
@@ -10,6 +11,16 @@ import pytest
 from problems import cone_lp
 
 pytestmark = pytest.mark.gpu
+
+
+def _reference_conelp(c, G, h, dims):
+    """the reference's own solvers.conelp(..., kktsolver='chol') run"""
+    from cvxopt import matrix, solvers
+    sol = solvers.conelp(matrix(c), matrix(G), matrix(h), dims, kktsolver="chol")
+    return {k: sol[k] if sol[k] is not None else np.nan for k in ("status", "iterations", "primal objective",
+            "dual objective", "x", "z", "gap", "primal infeasibility")}
+
+
 GOLD = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "config_runs.json")))
 
 
@@ -20,11 +31,10 @@ GOLD = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "
     ({"l": 0, "q": [], "s": [24]}, 30, 13),
     ({"l": 4, "q": [5], "s": [70]}, 50, 14),
 ])
-def test_device_conelp_matches_reference(ref, dims, n, seed):
+def test_device_conelp_matches_reference(ref_golden, dims, n, seed):
     import cvxopt_b200
-    from cvxopt import matrix, solvers
     c, G, h = cone_lp(n, dims, seed)
-    want = solvers.conelp(matrix(c), matrix(G), matrix(h), dims, kktsolver="chol")
+    want = ref_golden("conelp", lambda: _reference_conelp(c, G, h, dims))
     before = cvxopt_b200.launch_count()
     got = cvxopt_b200.conelp(c, G, h, dims)
     assert cvxopt_b200.launch_count() > before
@@ -37,15 +47,14 @@ def test_device_conelp_matches_reference(ref, dims, n, seed):
     np.testing.assert_allclose(got["primal infeasibility"], want["primal infeasibility"], rtol=1e-3, atol=1e-9)
 
 
-def test_device_conelp_infeasible_problem_gives_the_reference_certificate(ref):
+def test_device_conelp_infeasible_problem_gives_the_reference_certificate(ref_golden):
     """primal infeasible LP: x >= 1 and x <= 0 -> 'primal infeasible' after the same number of iterations"""
     import cvxopt_b200
-    from cvxopt import matrix, solvers
     G = np.array([[-1.0], [1.0]])
     h = np.array([-1.0, 0.0])
     c = np.array([1.0])
     dims = {"l": 2, "q": [], "s": []}
-    want = solvers.conelp(matrix(c), matrix(G), matrix(h), dims, kktsolver="chol")
+    want = ref_golden("conelp", lambda: _reference_conelp(c, G, h, dims))
     got = cvxopt_b200.conelp(c, G, h, dims)
     assert want["status"] == got["status"] == "primal infeasible"
     assert want["iterations"] == got["iterations"]

@@ -1,6 +1,7 @@
 """Nesterov-Todd scaling (SURVEY.md §8 rows a1, a2, f2): misc.compute_scaling / misc.update_scaling.
 
-CPU part: the oracle's restatements against the reference itself (oracle/_ref) — 'l', 'q' and 's' cones, mnl > 0.
+CPU part: the oracle's restatements against the reference itself (its stored results, tests/reference_results.py) —
+'l', 'q' and 's' cones, mnl > 0.
 GPU part: cvxopt_b200.scaling (device kernels: elementwise 'l', one CTA per 'q' cone, Cholesky + one-sided Jacobi
 SVD for 's') against the reference: d, di, v, beta, lambda elementwise; for 's' blocks the quantities that do not
 depend on the sign/order conventions of the SVD (r r', rti rti', rti' r = I, r' z r = diag(lambda)); and whole
@@ -10,6 +11,7 @@ import pytest
 
 import kkt_oracle as ko
 from problems import cone_dim, cone_lp, cone_point
+from reference_results import W_arrays, W_from_arrays
 
 CASES = [
     ({"l": 7, "q": [], "s": []}, 0),
@@ -74,29 +76,33 @@ def _compare_W(got, want, lam_got, lam_want, dims, mnl, tol=1e-11):
 
 
 @pytest.mark.parametrize("dims,mnl", CASES)
-def test_oracle_scaling_matches_reference(ref, dims, mnl):
-    from cvxopt import matrix, misc
+def test_oracle_scaling_matches_reference(ref_golden, dims, mnl):
     s, z, rng = _points(dims, mnl, seed=3)
+    sn, zn = _scaled_iterates(dims, mnl, rng)
+
+    def reference():
+        from cvxopt import matrix, misc
+        lam_r = matrix(0.0, (_nlam(dims, mnl), 1))
+        Wr = misc.compute_scaling(matrix(s), matrix(z), lam_r, dims, mnl if mnl else None)
+        out = dict(W_arrays(Wr, "W."), lam=+lam_r)
+        sr, zr = matrix(sn), matrix(zn)
+        misc.update_scaling(Wr, lam_r, sr, zr)
+        out.update(W_arrays(Wr, "Wu."), lamu=lam_r, s=sr, z=zr)
+        return out
+    want = ref_golden("scaling", reference)
     lam_o = np.zeros(_nlam(dims, mnl))
     Wo = ko.compute_scaling(s.copy(), z.copy(), lam_o, dims, mnl if mnl else None)
-    lam_r = matrix(0.0, (_nlam(dims, mnl), 1))
-    Wr = misc.compute_scaling(matrix(s), matrix(z), lam_r, dims, mnl if mnl else None)
-    _compare_W(Wo, _ref_W_to_np(Wr), lam_o, np.array(lam_r).ravel(), dims, mnl)
+    _compare_W(Wo, W_from_arrays(want, dims, "W."), lam_o, want["lam"].ravel(), dims, mnl)
     # update: both start from the SAME W (the scaled iterates are coordinates with respect to W, and the SVD's
     # sign conventions make W itself non-unique for 's' blocks)
-    sn, zn = _scaled_iterates(dims, mnl, rng)
     so, zo = sn.copy(), zn.copy()
-    Wo = _ref_W_to_np(Wr)
-    Wo["r"] = [np.asfortranarray(r) for r in Wo["r"]]
-    Wo["rti"] = [np.asfortranarray(r) for r in Wo["rti"]]
-    lam_o = np.array(lam_r).ravel().copy()
+    Wo = W_from_arrays(want, dims, "W.")
+    lam_o = want["lam"].ravel().copy()
     ko.update_scaling(Wo, lam_o, so, zo)
-    sr, zr = matrix(sn), matrix(zn)
-    misc.update_scaling(Wr, lam_r, sr, zr)
-    _compare_W(Wo, _ref_W_to_np(Wr), lam_o, np.array(lam_r).ravel(), dims, mnl)
+    _compare_W(Wo, W_from_arrays(want, dims, "Wu."), lam_o, want["lamu"].ravel(), dims, mnl)
     nlq = mnl + dims["l"] + sum(dims["q"])
-    np.testing.assert_allclose(so[:nlq], np.array(sr).ravel()[:nlq], rtol=1e-12)
-    np.testing.assert_allclose(zo[:nlq], np.array(zr).ravel()[:nlq], rtol=1e-12)
+    np.testing.assert_allclose(so[:nlq], want["s"].ravel()[:nlq], rtol=1e-12)
+    np.testing.assert_allclose(zo[:nlq], want["z"].ravel()[:nlq], rtol=1e-12)
 
 
 @pytest.mark.gpu

@@ -1,10 +1,12 @@
 """Batch of independent dense QPs solved in lock-step on the device (BASELINE config 4).
 
-    minimize 1/2 x'P x + q'x   subject to   G x <= h        (one 'l' cone of m rows, no A)
+    minimize 1/2 x'P x + q'x   subject to   G x <= h,  A x = b     (one 'l' cone of m rows, p rows of A)
 
 The per-problem algorithm is coneprog.coneqp restricted to dims={'l': m} (reference
 src/python/coneprog.py:1998-2547) — same start, stopping rule, Mehrotra steps — so every
-problem converges in the same number of iterations as `solvers.qp(P, q, G, h)` does.
+problem converges in the same number of iterations as `solvers.qp(P, q, G, h)` does, or, with
+equality constraints, as `solvers.qp(P, q, G, h, A, b)` does (its default KKT solver for this
+case, kktsolver='chol2', misc.py:1352-1567).  p = 0 (no A) is the default.
 The reference has no batch API; its counterpart is a Python loop over `solvers.qp`.
 """
 import ctypes as C
@@ -39,24 +41,49 @@ def _stack(P, q, G, h):
     return Pcm, q, Gcm, h, B, n, m
 
 
+def _stack_eq(A, b, B, n):
+    """-> contiguous (B,n,p) [= p x n column-major per problem], (B,p); (B,n,0), (B,0) without A"""
+    if A is None and b is None:
+        return np.zeros((B, n, 0)), np.zeros((B, 0)), 0
+    if A is None or b is None:
+        raise TypeError("A and b must be given together")
+    A = np.asarray(A, dtype=np.float64)
+    b = np.ascontiguousarray(np.asarray(b, dtype=np.float64))
+    if A.ndim != 3 or A.shape[0] != B or A.shape[2] != n:
+        raise TypeError("A must have shape (B, p, n)")
+    p = A.shape[1]
+    if b.shape != (B, p):
+        raise TypeError("b must have shape (B, p)")
+    return np.ascontiguousarray(np.transpose(A, (0, 2, 1))), b, p
+
+
 class QPBatch:
-    def __init__(self, nprob, n, m, device=0):
+    def __init__(self, nprob, n, m, device=0, p=0):
         self._lib = _lib.load()
         self._h = C.c_void_p()
-        self.B, self.n, self.m = int(nprob), int(n), int(m)
-        _lib.check(self._lib.cvxb_batch_create(C.byref(self._h), self.B, self.n, self.m, device), "batch")
+        self.B, self.n, self.m, self.p = int(nprob), int(n), int(m), int(p)
+        _lib.check(self._lib.cvxb_batch_create_eq(C.byref(self._h), self.B, self.n, self.m, self.p, device),
+                   "batch")
 
-    def load(self, P, q, G, h):
+    def load(self, P, q, G, h, A=None, b=None):
         Pcm, q, Gcm, h, B, n, m = _stack(P, q, G, h)
         if (B, n, m) != (self.B, self.n, self.m):
             raise TypeError("problem shapes do not match the batch")
+        Acm, b, p = _stack_eq(A, b, B, n)
+        if p != self.p:
+            raise TypeError("A has %d rows, the batch was created with p = %d" % (p, self.p))
         rc = self._lib.cvxb_batch_load(self._h, Pcm.ctypes.data, q.ctypes.data, Gcm.ctypes.data,
                                        h.ctypes.data, _lib.HOST)
         _lib.check(rc, "batch_load")
+        _lib.check(self._lib.cvxb_batch_load_eq(self._h, Acm.ctypes.data, b.ctypes.data, _lib.HOST), "batch_load_eq")
 
-    def load_ptr(self, P, q, G, h, space=_lib.DEVICE):
-        """raw addresses of already laid-out buffers (device-resident callers)"""
+    def load_ptr(self, P, q, G, h, space=_lib.DEVICE, A=None, b=None):
+        """raw addresses of already laid-out buffers (device-resident callers); A (p x n column-major per
+        problem) and b are required when p > 0"""
         _lib.check(self._lib.cvxb_batch_load(self._h, P, q, G, h, space), "batch_load")
+        if self.p > 0 and (not A or not b):
+            raise TypeError("A and b are required: the batch was created with p = %d" % self.p)
+        _lib.check(self._lib.cvxb_batch_load_eq(self._h, A, b, space), "batch_load_eq")
 
     def solve(self, **options):
         o = dict(DEFAULTS)
@@ -70,6 +97,7 @@ class QPBatch:
     def results(self):
         B, n, m = self.B, self.n, self.m
         x, s, z = np.zeros((B, n)), np.zeros((B, m)), np.zeros((B, m))
+        y = np.zeros((B, self.p))
         status = np.zeros(B, dtype=np.int32)
         iters = np.zeros(B, dtype=np.int32)
         pobj, dobj = np.zeros(B), np.zeros(B)
@@ -77,9 +105,23 @@ class QPBatch:
                                           status.ctypes.data, iters.ctypes.data, pobj.ctypes.data,
                                           dobj.ctypes.data, _lib.HOST)
         _lib.check(rc, "batch_results")
-        return {"x": x, "s": s, "z": z, "status": [STATUS[int(k)] for k in status],
+        _lib.check(self._lib.cvxb_batch_results_y(self._h, y.ctypes.data, _lib.HOST), "batch_results_y")
+        return {"x": x, "y": y, "s": s, "z": z, "status": [STATUS[int(k)] for k in status],
                 "status_code": status, "iterations": iters, "primal objective": pobj,
                 "dual objective": dobj}
+
+    def singular(self):
+        """per problem: True where S = P + G'G was singular at the starting point, so that S + A'A is factored
+        (the reference's kkt_chol2 'singular' branch)"""
+        flags = np.zeros(self.B, dtype=np.int32)
+        _lib.check(self._lib.cvxb_batch_singular(self._h, flags.ctypes.data), "batch_singular")
+        return flags.astype(bool)
+
+    def phase_ms(self):
+        """factorisation time of the last solve by phase (batch created with CVXB_BATCH_PHASE_MS=1)"""
+        ms = (C.c_double * 3)()
+        _lib.check(self._lib.cvxb_batch_phase_ms(self._h, ms), "batch_phase_ms")
+        return {"S_syrk_potrf_ms": ms[0], "trsm_ms": ms[1], "Kp_syrk_potrf_ms": ms[2]}
 
     def stats(self):
         ms, it = C.c_double(), C.c_int()
@@ -118,26 +160,30 @@ class QPBatchGroup:
     as ITS slowest problem is done.  Interleaved slices (problem i -> sub-batch i mod nsub) spread hard and easy
     problems evenly."""
 
-    def __init__(self, nprob, n, m, device=0, nsub=None):
+    def __init__(self, nprob, n, m, device=0, nsub=None, p=0):
         if nsub is None:
             # measured on B200 (profiles/r02h_batch_nsub.txt, n=512 m=1024): 512 problems 148 -> 142 ms with 2
             # sub-batches; 64 problems 25.0 -> 21.3 ms with 8
             nsub = int(__import__("os").environ.get("CVXB_BATCH_NSUB", "0")) or (
                 2 if nprob >= 256 else (max(1, min(8, nprob // 8)) if nprob >= 16 else 1))
         self.nsub = max(1, min(int(nsub), nprob))
-        self.B, self.n, self.m = int(nprob), int(n), int(m)
+        self.B, self.n, self.m, self.p = int(nprob), int(n), int(m), int(p)
         self.idx = [np.arange(r, self.B, self.nsub) for r in range(self.nsub)]
-        self.parts = [QPBatch(len(ix), n, m, device) for ix in self.idx]
+        self.parts = [QPBatch(len(ix), n, m, device, p) for ix in self.idx]
 
     def load_ptr_sliced(self, loader):
         """loader(part_index, indices, QPBatch) loads one sub-batch (device-resident callers)"""
         for r, (ix, b) in enumerate(zip(self.idx, self.parts)):
             loader(r, ix, b)
 
-    def load(self, P, q, G, h):
+    def load(self, P, q, G, h, A=None, b=None):
         P, q, G, h = (np.asarray(a) for a in (P, q, G, h))
-        for ix, b in zip(self.idx, self.parts):
-            b.load(P[ix], q[ix], G[ix], h[ix])
+        if A is not None:
+            A = np.asarray(A)
+        if b is not None:
+            b = np.asarray(b)
+        for ix, part in zip(self.idx, self.parts):
+            part.load(P[ix], q[ix], G[ix], h[ix], None if A is None else A[ix], None if b is None else b[ix])
 
     def solve(self, **options):
         if self.nsub == 1:
@@ -161,7 +207,7 @@ class QPBatchGroup:
 
     def results(self):
         B, n, m = self.B, self.n, self.m
-        out = {"x": np.zeros((B, n)), "s": np.zeros((B, m)), "z": np.zeros((B, m)),
+        out = {"x": np.zeros((B, n)), "y": np.zeros((B, self.p)), "s": np.zeros((B, m)), "z": np.zeros((B, m)),
                "status_code": np.zeros(B, dtype=np.int32), "iterations": np.zeros(B, dtype=np.int32),
                "primal objective": np.zeros(B), "dual objective": np.zeros(B)}
         for ix, b in zip(self.idx, self.parts):
@@ -169,6 +215,12 @@ class QPBatchGroup:
             for key in out:
                 out[key][ix] = r[key]
         out["status"] = [STATUS[int(k)] for k in out["status_code"]]
+        return out
+
+    def singular(self):
+        out = np.zeros(self.B, dtype=bool)
+        for ix, b in zip(self.idx, self.parts):
+            out[ix] = b.singular()
         return out
 
     def stats(self):
@@ -183,29 +235,31 @@ class QPBatchGroup:
             b.close()
 
 
-def qp_batch(P, q, G, h, device=0, nsub=None, **options):
-    """Solve B independent dense QPs on one GPU.  P (B,n,n), q (B,n), G (B,m,n), h (B,m).
+def qp_batch(P, q, G, h, A=None, b=None, device=0, nsub=None, **options):
+    """Solve B independent dense QPs on one GPU.  P (B,n,n), q (B,n), G (B,m,n), h (B,m), and optionally
+    equality constraints A (B,p,n), b (B,p) as in solvers.qp(P, q, G, h, A, b).
     nsub: number of concurrently solved sub-batches (QPBatchGroup); default 4 (1 for tiny batches)."""
     P = np.asarray(P)
     G = np.asarray(G)
-    b = QPBatchGroup(P.shape[0], P.shape[1], G.shape[1], device, nsub)
+    p = 0 if A is None else np.asarray(A).shape[1]
+    grp = QPBatchGroup(P.shape[0], P.shape[1], G.shape[1], device, nsub, p)
     try:
-        b.load(P, q, G, h)
+        grp.load(P, q, G, h, A, b)
         import time
         t0 = time.perf_counter()
-        b.solve(**options)
+        grp.solve(**options)
         wall = (time.perf_counter() - t0) * 1e3
-        out = b.results()
-        out.update(b.stats())
+        out = grp.results()
+        out.update(grp.stats())
         out["solve_wall_ms"] = wall
         return out
     finally:
-        b.close()
+        grp.close()
 
 
 # ---------------------------------------------------------------------------------------
 # multi-GPU: problems are independent -> shard them across ranks, no data-path collective.
-# One scatter of (P, q, G, h) from rank 0, one gather of (x, s, z, status, iters, objectives):
+# One scatter of (P, q, G, h[, A, b]) from rank 0, one gather of (x, s, z[, y], status, iters, objectives):
 # point-to-point send/recv groups over the process group (NCCL over NVLink on GPUs: ncclSend/ncclRecv
 # inside one group call; gloo in the CPU tests), exact shard sizes, nothing padded, and on GPUs nothing
 # bounces through the host: shards land in device memory and QPBatch loads them from there.
@@ -238,9 +292,11 @@ def _p2p(ops):
 
 
 def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interleaved", timings=None,
-                         nsub=None, **options):
+                         nsub=None, A=None, b=None, **options):
     """Rank 0 passes the full batch (other ranks pass None); every rank returns its shard's results and
     rank 0 additionally gets the gathered batch, in the original problem order, under key 'all'.
+    Equality constraints A (B,p,n), b (B,p) are optional (rank 0 only); `solver` (a stand-in for the
+    device solver) is then called as solver(P, q, G, h, A, b).
 
     `timings` (dict, optional) receives scatter_ms / solve_ms / gather_ms of this rank, measured with
     device events on the current stream (wall clock on CPU)."""
@@ -276,25 +332,26 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
                 self.t[name] = (time.perf_counter() - e0) * 1e3
     clk = _Clock()
 
-    meta = torch.zeros(3, dtype=torch.int64, device=dev)
+    meta = torch.zeros(4, dtype=torch.int64, device=dev)
     full = None
     if rank == 0:
-        # the batch in the layout QPBatch loads: column-major n x n / m x n per problem
+        # the batch in the layout QPBatch loads: column-major n x n / m x n / p x n per problem
         Pcm, qh, Gcm, hh, Btot, n, m = _stack(P, q, G, h)
-        meta = torch.tensor([Btot, n, m], dtype=torch.int64, device=dev)
-        full = [torch.from_numpy(a).to(dev) for a in (Pcm, qh, Gcm, hh)]       # one H2D of the whole batch
+        Acm, bh, p = _stack_eq(A, b, Btot, n)
+        meta = torch.tensor([Btot, n, m, p], dtype=torch.int64, device=dev)
+        full = [torch.from_numpy(a).to(dev) for a in ((Pcm, qh, Gcm, hh) + ((Acm, bh) if p else ()))]  # one H2D
     if world > 1:
         dist.broadcast(meta, 0, group=group)
-    Btot, n, m = (int(v) for v in meta.tolist())
+    Btot, n, m, p = (int(v) for v in meta.tolist())
     owners = shard_indices(Btot, world, sharding)
     mine = owners[rank]
     k = len(mine)
-    tails = [(n, n), (n,), (n, m), (m,)]
+    tails = [(n, n), (n,), (n, m), (m,)] + ([(n, p), (p,)] if p else [])
 
     # ---- setup (not data path): this rank's batch object = its device allocations ----
     local_dev = torch.cuda.current_device() if on_gpu else 0
     clk.start("setup_ms")
-    bobj = QPBatchGroup(k, n, m, local_dev, nsub) if (solver is None and k) else None
+    bobj = QPBatchGroup(k, n, m, local_dev, nsub, p) if (solver is None and k) else None
     clk.stop()
 
     # ---- scatter ----
@@ -323,11 +380,18 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
     # ---- solve ----
     clk.start("solve_ms")
     if solver is not None:
-        # stand-in (CPU tests): numpy in the public (B, m, n) layout
-        Pn, qn, Gn, hn = (t.cpu().numpy() for t in shard)
-        res = solver(np.transpose(Pn, (0, 2, 1)), qn, np.transpose(Gn, (0, 2, 1)), hn) if k else None
-        xs, ss, zs = ((torch.from_numpy(np.ascontiguousarray(res[key])).to(dev) if k
-                       else torch.empty((0, d), dtype=f64, device=dev)) for key, d in (("x", n), ("s", m), ("z", m)))
+        # stand-in (CPU tests): numpy in the public (B, m, n) / (B, p, n) layout
+        sh = [t.cpu().numpy() for t in shard]
+        args = [np.transpose(sh[0], (0, 2, 1)), sh[1], np.transpose(sh[2], (0, 2, 1)), sh[3]]
+        if p:
+            args += [np.transpose(sh[4], (0, 2, 1)), sh[5]]
+        res = solver(*args) if k else None
+
+        def rows(key, d):
+            if not k or not d:
+                return torch.empty((k, d), dtype=f64, device=dev)
+            return torch.from_numpy(np.ascontiguousarray(res[key], dtype=np.float64)).to(dev)
+        xs, ss, zs, ys = rows("x", n), rows("s", m), rows("z", m), rows("y", p)
         sc = torch.zeros((k, 4), dtype=f64, device=dev)
         if k:
             for j, key in enumerate(("status_code", "iterations", "primal objective", "dual objective")):
@@ -337,36 +401,40 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
         xs = torch.empty((k, n), dtype=f64, device=dev)
         ss = torch.empty((k, m), dtype=f64, device=dev)
         zs = torch.empty((k, m), dtype=f64, device=dev)
+        ys = torch.empty((k, p), dtype=f64, device=dev)
         sc = torch.zeros((k, 4), dtype=f64, device=dev)
         stats = {}
         if k:
-            b = bobj
+            grp = bobj
             try:
                 # shards are already in device memory: straight into the sub-batches, no host bounce
                 keepalive = []
 
                 def loader(r, ix, part):
                     it = torch.from_numpy(ix).to(dev)
-                    sl = [t.index_select(0, it) for t in shard] if b.nsub > 1 else shard
+                    sl = [t.index_select(0, it) for t in shard] if grp.nsub > 1 else shard
                     keepalive.append(sl)
                     # the library copies on the sub-batch's own stream: the slices (written on torch's current
                     # stream) must be complete before it reads them
                     torch.cuda.current_stream().synchronize()
-                    part.load_ptr(sl[0].data_ptr(), sl[1].data_ptr(), sl[2].data_ptr(), sl[3].data_ptr(), _lib.DEVICE)
+                    eq = dict(A=sl[4].data_ptr(), b=sl[5].data_ptr()) if p else {}
+                    part.load_ptr(sl[0].data_ptr(), sl[1].data_ptr(), sl[2].data_ptr(), sl[3].data_ptr(), _lib.DEVICE,
+                                  **eq)
                 tw = time.perf_counter()
-                b.load_ptr_sliced(loader)
+                grp.load_ptr_sliced(loader)
                 del keepalive
                 clk.t["solve_load_wall_ms"] = (time.perf_counter() - tw) * 1e3
                 tw = time.perf_counter()
-                b.solve(**options)
+                grp.solve(**options)
                 clk.t["solve_ipm_wall_ms"] = (time.perf_counter() - tw) * 1e3
                 tw = time.perf_counter()
-                for ix, part in zip(b.idx, b.parts):
+                for ix, part in zip(grp.idx, grp.parts):
                     kk = len(ix)
                     it = torch.from_numpy(ix).to(dev)
                     px = torch.empty((kk, n), dtype=f64, device=dev)
                     ps = torch.empty((kk, m), dtype=f64, device=dev)
                     pz = torch.empty((kk, m), dtype=f64, device=dev)
+                    py = torch.empty((kk, p), dtype=f64, device=dev)
                     status = np.zeros(kk, dtype=np.int32); iters = np.zeros(kk, dtype=np.int32)
                     pobj, dobj = np.zeros(kk), np.zeros(kk)
                     lib = part._lib
@@ -375,29 +443,33 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
                                                       None, None, _lib.DEVICE), "batch_results")
                     _lib.check(lib.cvxb_batch_results(part._h, None, None, None, status.ctypes.data, iters.ctypes.data,
                                                       pobj.ctypes.data, dobj.ctypes.data, _lib.HOST), "batch_results")
+                    if p:
+                        _lib.check(lib.cvxb_batch_results_y(part._h, py.data_ptr(), _lib.DEVICE), "batch_results_y")
+                        ys.index_copy_(0, it, py)
                     xs.index_copy_(0, it, px); ss.index_copy_(0, it, ps); zs.index_copy_(0, it, pz)
                     sc.index_copy_(0, it, torch.from_numpy(np.stack(
                         [status.astype(np.float64), iters.astype(np.float64), pobj, dobj], axis=1)).to(dev))
-                stats = b.stats()
+                stats = grp.stats()
                 torch.cuda.synchronize()
                 clk.t["solve_collect_wall_ms"] = (time.perf_counter() - tw) * 1e3
             except BaseException:
-                b.close()
+                grp.close()
                 raise
     del shard
     clk.stop()
 
     # ---- gather ----
     clk.start("gather_ms")
-    local = [xs, ss, zs, sc]
+    local = [xs, ss, zs, sc] + ([ys] if p else [])
+    widths = (n, m, m, 4) + ((p,) if p else ())
     gathered = None
     if rank == 0:
-        outs = [torch.empty((Btot, d), dtype=f64, device=dev) for d in (n, m, m, 4)]
+        outs = [torch.empty((Btot, d), dtype=f64, device=dev) for d in widths]
         ops, bufs = [], {}
         for r in range(1, world):
             kr = len(owners[r])
             if kr:
-                bufs[r] = [torch.empty((kr, d), dtype=f64, device=dev) for d in (n, m, m, 4)]
+                bufs[r] = [torch.empty((kr, d), dtype=f64, device=dev) for d in widths]
                 ops += [dist.P2POp(dist.irecv, t, r, group) for t in bufs[r]]
         _p2p(ops)
         bufs[0] = local
@@ -415,14 +487,15 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
         timings.update(clk.t)
 
     scn = sc.cpu().numpy()
-    res = {"x": xs.cpu().numpy(), "s": ss.cpu().numpy(), "z": zs.cpu().numpy(),
+    res = {"x": xs.cpu().numpy(), "y": ys.cpu().numpy(), "s": ss.cpu().numpy(), "z": zs.cpu().numpy(),
            "status_code": scn[:, 0].astype(np.int32), "iterations": scn[:, 1].astype(np.int32),
            "primal objective": scn[:, 2].copy(), "dual objective": scn[:, 3].copy(), "indices": mine}
     res.update(stats)
     res["status"] = [STATUS[int(c)] for c in res["status_code"]]
     if rank == 0:
         g = gathered
-        res["all"] = {"x": g[0], "s": g[1], "z": g[2], "status_code": g[3][:, 0].astype(np.int64),
+        res["all"] = {"x": g[0], "y": g[4] if p else np.zeros((Btot, 0)), "s": g[1], "z": g[2],
+                      "status_code": g[3][:, 0].astype(np.int64),
                       "iterations": g[3][:, 1].astype(np.int64), "primal objective": g[3][:, 2].copy(),
                       "dual objective": g[3][:, 3].copy(),
                       "status": [STATUS[int(c)] for c in g[3][:, 0]]}

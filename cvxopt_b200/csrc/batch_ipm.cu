@@ -1,6 +1,6 @@
 // Device-resident primal-dual interior-point method for a BATCH of independent dense QPs
 //
-//      minimize  1/2 x'P x + q'x    subject to  G x + s = h,  s >= 0          ('l' cone, no A)
+//      minimize  1/2 x'P x + q'x    subject to  G x + s = h,  s >= 0,  A x = b      ('l' cone, p >= 0 rows of A)
 //
 // run in lock-step, one problem per CTA-group, with per-problem convergence masks
 // (BASELINE config 4; the reference has no batch API — its counterpart is a Python loop over
@@ -11,7 +11,13 @@
 // (misc.py:450-464).  Every KKT solve is the same path as cvxb_kkt_*: fused-scaling SYRK,
 // Cholesky, GEMV/TRSV — here batched over the problems through blockIdx.z / blockIdx.y.
 // Nothing leaves the device between iterations except one int ("how many are done").
-#include "cone.cuh"
+//
+// Equality constraints (p > 0) are eliminated as the reference's default KKT solver for this case does,
+// misc.kkt_chol2 (misc.py:1352-1567): S = P + G' D^-2 G = L L', Asct = L^{-1} A', Kp = Asct' Asct = Lp Lp'.
+// A problem whose S is singular at the starting point (W = I) factors S + A'A from then on (misc.py:1421-1461);
+// per problem, through a 0/1 weight vector of length p (`wsing`) applied inside the batched GEMM / GEMV.
+#include "kkt_internal.cuh"
+#include <algorithm>
 #include <cstdlib>
 
 using namespace cvxb;
@@ -21,7 +27,9 @@ namespace {
 struct Scal {                       // per-problem scalars, device resident
     double resx0, resz0, gap, mu, sigma, eta, step, dsdz;
     double xPxq, xq, resx, resz, zrz, pcost, dcost, relgap, pres, dres;
+    double resy0, resy, yry;                 // equality constraints: max(1, ||b||), ||A x - b||, y'(A x - b)
     int relgap_valid, done, iters, status;   // status: 0 running, 1 optimal, 2 maxiters, 3 singular
+    int singular, pad_;                      // singular: S + A'A is factored (kkt_chol2's F['singular'])
 };
 
 __device__ __forceinline__ double block_sum(double v, double *sh) {
@@ -54,9 +62,10 @@ __device__ __forceinline__ double block_min(double v, double *sh) {
 }
 
 struct Ptrs {
-    int n, m;
-    const double *q, *h;
+    int n, m, neq;                  // neq: rows of A (p)
+    const double *q, *h, *beq;
     double *x, *s, *z, *rx, *rz, *dx, *ds, *dz, *lmbda, *lmbdasq, *d, *di, *di2, *ws3, *bzp;
+    double *y, *ry, *dy, *wsing;    // p-vectors (wsing: 1 where S + A'A is factored, else 0)
     Scal *sc;
 };
 #define PB_SETUP                                                  \
@@ -78,8 +87,15 @@ __global__ void k_init_rhs(Ptrs p) {
     }
     nq = block_sum(nq, sh);
     nh = block_sum(nh, sh);
+    double nb = 0;
+    if (p.neq > 0) {                                    // dy = b
+        const long long op = (long long)b * p.neq;
+        for (int i = tid; i < p.neq; i += nt) { double v = p.beq[op + i]; p.dy[op + i] = v; nb += v * v; }
+        nb = block_sum(nb, sh);
+    }
     if (tid == 0) {
         S.resx0 = fmax(1.0, sqrt(nq));                  // :1998
+        S.resy0 = fmax(1.0, sqrt(nb));                  // :1999
         S.resz0 = fmax(1.0, sqrt(nh));                  // :2000 (snrm2 == 2-norm for 'l')
         S.done = 0; S.iters = 0; S.status = 0; S.sigma = 0; S.eta = 0; S.step = 0;
     }
@@ -95,6 +111,8 @@ __global__ void k_init_point(Ptrs p) {
     PB_SETUP
     double ns = 0, mins = INFINITY;
     for (int i = tid; i < p.n; i += nt) p.x[on + i] = p.dx[on + i];
+    const long long op = (long long)b * p.neq;
+    for (int i = tid; i < p.neq; i += nt) p.y[op + i] = p.dy[op + i];
     for (int i = tid; i < p.m; i += nt) {
         double zv = p.bzp[om + i];      // solve leaves W*uz in bzp
         p.z[om + i] = zv;
@@ -120,12 +138,14 @@ __global__ void k_init_point(Ptrs p) {
     gap = block_sum(gap, sh);
     if (tid == 0) S.gap = gap;
 }
-// rx = q  (then rx += P x by GEMV)
+// rx = q  (then rx += P x by GEMV); ry = b (then ry := A x - ry)
 __global__ void k_res_begin(Ptrs p) {
     PB_SETUP
     (void)sh; (void)S;
     for (int i = tid; i < p.n; i += nt) p.rx[on + i] = p.q[on + i];
     for (int i = tid; i < p.m; i += nt) p.rz[om + i] = p.s[om + i] - p.h[om + i];      // :2183-2184
+    const long long op = (long long)b * p.neq;
+    for (int i = tid; i < p.neq; i += nt) p.ry[op + i] = p.beq[op + i];                 // :2178
 }
 // f0 pieces once rx = P x + q   (:2172)
 __global__ void k_res_dots(Ptrs p) {
@@ -143,16 +163,23 @@ __global__ void k_stats(Ptrs p, int iter, int maxiters, double abstol, double re
     for (int i = tid; i < p.n; i += nt) { double v = p.rx[on + i]; rx2 += v * v; }
     for (int i = tid; i < p.m; i += nt) { double v = p.rz[om + i]; rz2 += v * v; zrz += p.z[om + i] * v; }
     rx2 = block_sum(rx2, sh); rz2 = block_sum(rz2, sh); zrz = block_sum(zrz, sh);
+    double ry2 = 0, yry = 0;
+    if (p.neq > 0) {
+        const long long op = (long long)b * p.neq;
+        for (int i = tid; i < p.neq; i += nt) { double v = p.ry[op + i]; ry2 += v * v; yry += p.y[op + i] * v; }
+        ry2 = block_sum(ry2, sh); yry = block_sum(yry, sh);
+    }
     if (tid == 0) {
         if (!S.done) {
             const double f0 = 0.5 * (S.xPxq + S.xq);
             S.resx = sqrt(rx2); S.resz = sqrt(rz2); S.zrz = zrz;
+            S.resy = sqrt(ry2); S.yry = yry;
             S.pcost = f0;
-            S.dcost = f0 + zrz - S.gap;
+            S.dcost = (p.neq > 0 ? f0 + yry : f0) + zrz - S.gap;
             if (S.pcost < 0.0) { S.relgap = S.gap / -S.pcost; S.relgap_valid = 1; }
             else if (S.dcost > 0.0) { S.relgap = S.gap / S.dcost; S.relgap_valid = 1; }
             else { S.relgap = 0.0; S.relgap_valid = 0; }
-            S.pres = S.resz / S.resz0;
+            S.pres = p.neq > 0 ? fmax(S.resy / S.resy0, S.resz / S.resz0) : S.resz / S.resz0;
             S.dres = S.resx / S.resx0;
             const bool opt = S.pres <= feastol && S.dres <= feastol &&
                              (S.gap <= abstol || (S.relgap_valid && S.relgap <= reltol));
@@ -168,18 +195,20 @@ __global__ void k_stats(Ptrs p, int iter, int maxiters, double abstol, double re
 // ---- compaction of finished problems ----
 // The lock-step loop launches every batched kernel over the first `Bact` slots.  When problems finish, each finished
 // slot below the new active count trades places with an active slot from the tail: everything a problem owns between
-// iterations (P, G, its 17 vectors, its scalars; K / inv / info are rebuilt every iteration) is swapped, so the active
+// iterations (P, G, A, its 17 + 5 vectors, its scalars; K / inv / info / Asct / Kp are rebuilt every iteration) is swapped,
+// so the active
 // problems stay a contiguous prefix and finished ones keep their final iterates in the tail.  ~6.3 MB per swap at
-// n=512, m=1024, at most one swap per problem per solve.
+// n=512, m=1024 (p = 0), at most one swap per problem per solve.
 struct SwapArgs {
-    double *P, *G, *vecs; Scal *sc;
-    long long sP, sG;
-    int n, me, Btot;
+    double *P, *G, *vecs, *A, *veq; Scal *sc;
+    long long sP, sG, sA;
+    int n, me, neq, Btot;
 };
 __global__ void k_swap_slots(SwapArgs a, const int *pairs) {
     const int i = pairs[2 * blockIdx.y], j = pairs[2 * blockIdx.y + 1];
     const long long eP = a.sP, eG = a.sG, eN = 4LL * a.n, eM = 13LL * a.me, eS = (long long)(sizeof(Scal) / sizeof(double));
-    const long long total = eP + eG + eN + eM + eS;
+    const long long eA = a.sA, eQ = 5LL * a.neq;          // both 0 without equality constraints
+    const long long total = eP + eG + eN + eM + eS + eA + eQ;
     for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
         double *x, *y;
         long long r = e;
@@ -193,9 +222,15 @@ __global__ void k_swap_slots(SwapArgs a, const int *pairs) {
             const long long arr = r / a.me, k = r % a.me;
             double *base = a.vecs + 4LL * a.Btot * a.n + arr * (long long)a.Btot * a.me;
             x = base + (long long)i * a.me + k; y = base + (long long)j * a.me + k;
-        } else {
-            r -= eM;
+        } else if ((r -= eM) < eS) {
             x = reinterpret_cast<double *>(a.sc + i) + r; y = reinterpret_cast<double *>(a.sc + j) + r;
+        } else if ((r -= eS) < eA) {
+            x = a.A + i * a.sA + r; y = a.A + j * a.sA + r;
+        } else {
+            r -= eA;
+            const long long arr = r / a.neq, k = r % a.neq;
+            double *base = a.veq + arr * (long long)a.Btot * a.neq;
+            x = base + (long long)i * a.neq + k; y = base + (long long)j * a.neq + k;
         }
         const double t = *x; *x = *y; *y = t;
     }
@@ -208,6 +243,30 @@ __global__ void k_unpermute_rows(const double *in, double *out, const int *perm,
     for (int k = threadIdx.x; k < len; k += blockDim.x) dst[k] = src[k];
 }
 static_assert(sizeof(Scal) % sizeof(double) == 0, "Scal is swapped as doubles");
+
+// kkt_chol2's first factorisation (misc.py:1421-1447): a problem whose S did not factor at the starting point is
+// flagged, and S + A'A is factored for it from then on.  info: one int per problem from the Cholesky of S.
+__global__ void k_flag_singular(Ptrs p, const int *info, int *nsing) {
+    const int b = blockIdx.x;
+    if (info[b] <= 0) return;
+    const long long op = (long long)b * p.neq;
+    for (int k = threadIdx.x; k < p.neq; k += blockDim.x) p.wsing[op + k] = 1.0;
+    if (threadIdx.x == 0) { p.sc[b].singular = 1; atomicAdd(nsing, 1); }
+}
+// a failed Cholesky of Kp counts as a failed factorisation of the problem (the reference raises either way)
+__global__ void k_fold_info(const int *infop, int *info, int n, int B) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b < B && info[b] <= 0 && infop[b] > 0) info[b] = n + infop[b];
+}
+// Asct := A'  (p x n, ld lda  ->  n x p, ld ldas), every problem of the batch (blockIdx.y)
+__global__ void k_transpose_A(const double *A, long long lda, long long sA, double *At, long long ldas, long long sAt,
+                              int n, int neq) {
+    const long long b = blockIdx.y, tot = (long long)n * neq;
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < tot; e += (long long)gridDim.x * blockDim.x) {
+        const long long i = e % n, k = e / n;
+        At[b * sAt + i + k * ldas] = A[b * sA + k + i * lda];
+    }
+}
 // NT scaling at iteration 0 (misc.py:284-287) and lambda^2 (:2244)
 __global__ void k_scaling(Ptrs p, int first) {
     PB_SETUP
@@ -234,6 +293,8 @@ __global__ void k_dir_prep(Ptrs p, int i) {
     (void)sh;
     const double sm = S.sigma * S.mu, c = -1.0 + S.eta;
     for (int k = tid; k < p.n; k += nt) p.dx[on + k] = c * p.rx[on + k];
+    const long long op = (long long)b * p.neq;
+    for (int k = tid; k < p.neq; k += nt) p.dy[op + k] = c * p.ry[op + k];
     for (int k = tid; k < p.m; k += nt) {
         double ds = -p.lmbdasq[om + k] + sm;
         if (i == 1) ds -= p.ws3[om + k];                 // Mehrotra correction
@@ -284,6 +345,8 @@ __global__ void k_update(Ptrs p, const int *info, int iter) {
     }
     const double step = S.step;
     for (int k = tid; k < p.n; k += nt) p.x[on + k] += step * p.dx[on + k];
+    const long long op = (long long)b * p.neq;
+    for (int k = tid; k < p.neq; k += nt) p.y[op + k] += step * p.dy[op + k];
     double gap = 0;
     for (int k = tid; k < p.m; k += nt) {
         const double l = p.lmbda[om + k];
@@ -311,6 +374,20 @@ struct cvxb_batch {
     long long sG = 0, sP = 0, sK = 0, sInv = 0;
     int nblk = 0;
     double *P = nullptr, *G = nullptr, *q = nullptr, *h = nullptr;
+    // equality constraints A x = b (p = neq rows; nothing is allocated when p = 0)
+    int neq = 0;
+    long long lda = 0, ldkp = 0, sA = 0, sAs = 0, sKp = 0, sInvp = 0;
+    double *A = nullptr;             // p x n per problem (ld lda)
+    double *Asct = nullptr;          // n x p per problem (ld ldk): L^{-1} A'
+    double *Kp = nullptr, *invp = nullptr;   // p x p per problem (ld ldkp): Asct' Asct, then its Cholesky factor
+    double *veq = nullptr;           // p-vectors: b y ry dy wsing
+    int *d_infop = nullptr, *d_nsing = nullptr;
+    int nsing = 0;                   // problems flagged singular at the start of the last solve
+    bool eq_loaded = false;
+    // CVXB_BATCH_PHASE_MS=1 (read at create): time the factorisations' phases, synchronising after each one
+    bool time_phases = false;
+    double phase_ms[3] = {0, 0, 0};  // S: SYRK + Cholesky; TRSM (Asct); Kp: SYRK + Cholesky
+    cudaEvent_t ph[4] = {nullptr, nullptr, nullptr, nullptr};
     double *K = nullptr, *inv = nullptr, *panel = nullptr, *gemv_ws = nullptr;
     double *vecs = nullptr;          // all n- and m-vectors
     Ptrs p;
@@ -338,8 +415,91 @@ struct cvxb_batch {
 
 namespace {
 
-int batch_factor(cvxb_batch *b) {
+void phase_mark(cvxb_batch *b, int k) {
+    if (b->time_phases) cudaEventRecord(b->ph[k], b->st);
+}
+// adds the time between marks k and k+1 to phase k (synchronises: timing runs only)
+void phase_add(cvxb_batch *b, int k) {
+    if (!b->time_phases) return;
+    float t = 0;
+    cudaEventSynchronize(b->ph[k + 1]);
+    if (cudaEventElapsedTime(&t, b->ph[k], b->ph[k + 1]) == cudaSuccess) b->phase_ms[k] += t;
+    cudaGetLastError();
+}
+
+// K := P + G' diag(di)^2 G (+ A' diag(wsing) A where flagged) and its Cholesky factor; d_info per problem
+int factor_S(cvxb_batch *b, bool i8) {
     cudaStream_t st = b->st;
+    if (i8) {
+        CVXB_TRY(ozaki_syrk(b->n, b->m, b->G, b->ldg, b->p.di, b->P, b->ldp, 1.0, b->K, b->ldk, 9, 0,
+                            b->oz_work, nullptr, st));
+    } else {
+        GemmDesc g;
+        g.M = b->n; g.N = b->n; g.K = b->m;
+        g.X = b->G; g.ldx = (int)b->ldg; g.x_kmajor = true; g.sX = b->sG;
+        g.Y = b->G; g.ldy = (int)b->ldg; g.y_kmajor = true; g.sY = b->sG;
+        g.w = b->p.di2; g.sW = b->m;
+        g.D = b->P; g.ldd = (int)b->ldp; g.sD = b->sP; g.beta = 1.0;
+        g.C = b->K; g.ldc = (int)b->ldk; g.sC = b->sK;
+        g.lower_only = true; g.batch = b->Bact;
+        if (b->B == 1) g.splitk_ws = b->cw.splitk_ws;
+        CVXB_TRY(dmma_gemm(g, st));
+    }
+    if (b->nsing > 0) {
+        // K += A' diag(wsing) A: adds A'A to the flagged problems' S and exactly zero to the others (misc.py:1452-1454)
+        GemmDesc g;
+        g.M = b->n; g.N = b->n; g.K = b->neq;
+        g.X = b->A; g.ldx = (int)b->lda; g.x_kmajor = true; g.sX = b->sA;
+        g.Y = b->A; g.ldy = (int)b->lda; g.y_kmajor = true; g.sY = b->sA;
+        g.w = b->p.wsing; g.sW = b->neq;
+        g.D = b->K; g.ldd = (int)b->ldk; g.sD = b->sK; g.beta = 1.0;
+        g.C = b->K; g.ldc = (int)b->ldk; g.sC = b->sK;
+        g.lower_only = true; g.batch = b->Bact;
+        CVXB_TRY(dmma_gemm(g, st));
+    }
+    if (b->B == 1) {
+        CVXB_TRY(potrf_lower(b->n, b->K, (int)b->ldk, b->inv, b->cw, st));
+        CVXB_CUDA(cudaMemcpyAsync(b->d_info, b->cw.d_info, sizeof(int), cudaMemcpyDeviceToDevice, st));
+    } else {
+        CVXB_TRY(potrf_lower_batched(b->n, b->K, (int)b->ldk, b->sK, b->inv, b->sInv, b->Bact, b->d_info,
+                                     b->panel, (b->n + 1) & ~1, st));
+    }
+    return 0;
+}
+
+// Asct := L^{-1} A',  Kp := Asct' Asct = Lp Lp'  (misc.py:1464-1472); a failed Kp pivot is folded into d_info
+int factor_eq(cvxb_batch *b) {
+    cudaStream_t st = b->st;
+    const int n = b->n, pe = b->neq, B = b->Bact;
+    phase_mark(b, 1);
+    {
+        const long long tot = (long long)n * pe;
+        const unsigned gx = (unsigned)((tot + 255) / 256 < 64 ? (tot + 255) / 256 : 64);
+        k_transpose_A<<<dim3(gx, B), 256, 0, st>>>(b->A, b->lda, b->sA, b->Asct, b->ldk, b->sAs, n, pe);
+        count_launch();
+    }
+    CVXB_TRY(trsm_lower_left(n, b->K, b->ldk, b->inv, b->Asct, b->ldk, pe, st, B, b->sK, b->sInv, b->sAs));
+    phase_mark(b, 2);
+    GemmDesc g;
+    g.M = pe; g.N = pe; g.K = n;
+    g.X = b->Asct; g.ldx = (int)b->ldk; g.x_kmajor = true; g.sX = b->sAs;
+    g.Y = b->Asct; g.ldy = (int)b->ldk; g.y_kmajor = true; g.sY = b->sAs;
+    g.C = b->Kp; g.ldc = (int)b->ldkp; g.sC = b->sKp;
+    g.lower_only = true; g.batch = B;
+    CVXB_TRY(dmma_gemm(g, st));
+    CVXB_TRY(potrf_lower_batched(pe, b->Kp, (int)b->ldkp, b->sKp, b->invp, b->sInvp, B, b->d_infop, b->panel,
+                                 (int)b->ldkp, st));
+    k_fold_info<<<(B + 255) / 256, 256, 0, st>>>(b->d_infop, b->d_info, n, B);
+    count_launch();
+    CVXB_LAUNCH_CHECK();
+    phase_mark(b, 3);
+    phase_add(b, 1);
+    phase_add(b, 2);
+    return 0;
+}
+
+// first: the factorisation at the starting point (W = I), where kkt_chol2 decides which problems are singular
+int batch_factor(cvxb_batch *b, bool first = false) {
     bool i8 = b->B == 1 && b->m > 0 && (b->i8_mode == 2 || (b->i8_mode == 1 && b->n >= 4096 && b->m >= 8192));
     if (i8) {
         // K = P + G' diag(di)^2 G from nine int8 slices per entry (fp64-accurate, ~1.8x the DMMA SYRK);
@@ -360,41 +520,45 @@ int batch_factor(cvxb_batch *b) {
         }
     }
     b->syrk_path = i8 ? 2 : 1;
-    if (i8) {
-        CVXB_TRY(ozaki_syrk(b->n, b->m, b->G, b->ldg, b->p.di, b->P, b->ldp, 1.0, b->K, b->ldk, 9, 0,
-                            b->oz_work, nullptr, st));
-        CVXB_TRY(potrf_lower(b->n, b->K, (int)b->ldk, b->inv, b->cw, st));
-        CVXB_CUDA(cudaMemcpyAsync(b->d_info, b->cw.d_info, sizeof(int), cudaMemcpyDeviceToDevice, st));
-        return 0;
+    phase_mark(b, 0);
+    CVXB_TRY(factor_S(b, i8));
+    if (b->neq > 0 && first) {
+        CVXB_CUDA(cudaMemsetAsync(b->d_nsing, 0, sizeof(int), b->st));
+        k_flag_singular<<<b->Bact, 128, 0, b->st>>>(b->p, b->d_info, b->d_nsing);
+        count_launch();
+        CVXB_CUDA(cudaMemcpyAsync(&b->nsing, b->d_nsing, sizeof(int), cudaMemcpyDeviceToHost, b->st));
+        CVXB_CUDA(cudaStreamSynchronize(b->st));
+        if (b->nsing > 0) CVXB_TRY(factor_S(b, i8));
     }
-    GemmDesc g;
-    g.M = b->n; g.N = b->n; g.K = b->m;
-    g.X = b->G; g.ldx = (int)b->ldg; g.x_kmajor = true; g.sX = b->sG;
-    g.Y = b->G; g.ldy = (int)b->ldg; g.y_kmajor = true; g.sY = b->sG;
-    g.w = b->p.di2; g.sW = b->m;
-    g.D = b->P; g.ldd = (int)b->ldp; g.sD = b->sP; g.beta = 1.0;
-    g.C = b->K; g.ldc = (int)b->ldk; g.sC = b->sK;
-    g.lower_only = true; g.batch = b->Bact;
-    if (b->B == 1) g.splitk_ws = b->cw.splitk_ws;
-    CVXB_TRY(dmma_gemm(g, st));
-    if (b->B == 1) {
-        CVXB_TRY(potrf_lower(b->n, b->K, (int)b->ldk, b->inv, b->cw, st));
-        CVXB_CUDA(cudaMemcpyAsync(b->d_info, b->cw.d_info, sizeof(int), cudaMemcpyDeviceToDevice, st));
-    } else {
-        CVXB_TRY(potrf_lower_batched(b->n, b->K, (int)b->ldk, b->sK, b->inv, b->sInv, b->Bact, b->d_info,
-                                     b->panel, (b->n + 1) & ~1, st));
-    }
+    phase_mark(b, 1);
+    phase_add(b, 0);
+    if (b->neq > 0) CVXB_TRY(factor_eq(b));
     return 0;
 }
 
-// (dx, bzp) := solution of the reduced KKT system; on entry dx = bx, bzp = W^{-T} bz
+// (dx, dy, bzp) := solution of the reduced KKT system; on entry dx = bx, dy = by, bzp = W^{-T} bz
 int batch_solve(cvxb_batch *b) {
     cudaStream_t st = b->st;
-    const int n = b->n, m = b->m, B = b->Bact;
+    const int n = b->n, m = b->m, B = b->Bact, pe = b->neq;
     GemvBatch gt; gt.batch = B; gt.sA = b->sG; gt.sw = m; gt.sx = m; gt.sy = n;
     // x := x + G' (di .* bzp)
     CVXB_TRY(gemv_t(m, n, b->G, b->ldg, b->p.di, b->p.bzp, 1.0, 1.0, b->p.dx, st, gt));
-    CVXB_TRY(potrs_lower(n, b->K, (int)b->ldk, b->inv, b->p.dx, b->cw, st, B, b->sK, b->sInv, n));
+    if (pe == 0) {
+        CVXB_TRY(potrs_lower(n, b->K, (int)b->ldk, b->inv, b->p.dx, b->cw, st, B, b->sK, b->sInv, n));
+    } else {
+        // kkt_chol2's solve (misc.py:1526-1558)
+        if (b->nsing > 0) {       // x += A' by where S + A'A is factored
+            GemvBatch ga; ga.batch = B; ga.sA = b->sA; ga.sw = pe; ga.sx = pe; ga.sy = n;
+            CVXB_TRY(gemv_t(pe, n, b->A, b->lda, b->p.wsing, b->p.dy, 1.0, 1.0, b->p.dx, st, ga));
+        }
+        CVXB_TRY(trsv_lower(n, b->K, (int)b->ldk, b->inv, b->p.dx, false, b->cw, st, B, b->sK, b->sInv, n));
+        GemvBatch gyt; gyt.batch = B; gyt.sA = b->sAs; gyt.sx = n; gyt.sy = pe;       // y := Asct' x - y
+        CVXB_TRY(gemv_t(n, pe, b->Asct, b->ldk, nullptr, b->p.dx, 1.0, -1.0, b->p.dy, st, gyt));
+        CVXB_TRY(potrs_lower(pe, b->Kp, (int)b->ldkp, b->invp, b->p.dy, b->cw, st, B, b->sKp, b->sInvp, pe));
+        GemvBatch gyn; gyn.batch = B; gyn.sA = b->sAs; gyn.sx = pe; gyn.sy = n;       // x -= Asct y
+        CVXB_TRY(gemv_n(n, pe, b->Asct, b->ldk, nullptr, b->p.dy, -1.0, 1.0, b->p.dx, b->gemv_ws, st, gyn));
+        CVXB_TRY(trsv_lower(n, b->K, (int)b->ldk, b->inv, b->p.dx, true, b->cw, st, B, b->sK, b->sInv, n));
+    }
     // bzp := di .* (G x) - bzp
     GemvBatch gn; gn.batch = B; gn.sA = b->sG; gn.sw = m; gn.sx = n; gn.sy = m;
     CVXB_TRY(gemv_n(m, n, b->G, b->ldg, b->p.di, b->p.dx, 1.0, -1.0, b->p.bzp, b->gemv_ws, st, gn));
@@ -406,7 +570,13 @@ int batch_solve(cvxb_batch *b) {
 extern "C" {
 
 int cvxb_batch_create(cvxb_batch **out, int nprob, int n, int m, int device) {
+    return cvxb_batch_create_eq(out, nprob, n, m, 0, device);
+}
+
+int cvxb_batch_create_eq(cvxb_batch **out, int nprob, int n, int m, int p, int device) {
     if (!out || nprob <= 0 || n <= 0 || m < 0) { set_error("batch_create: bad sizes"); return CVXB_E_ARG; }
+    if (p < 0 || p > n) { set_error("batch_create: need 0 <= p <= n (p = %d, n = %d)", p, n); return CVXB_E_ARG; }
+    if (p > 0 && m == 0) { set_error("batch_create: equality constraints need m > 0"); return CVXB_E_ARG; }
     *out = nullptr;
     int cnt = 0;
     if (cudaGetDeviceCount(&cnt) != cudaSuccess || cnt == 0) {
@@ -417,7 +587,7 @@ int cvxb_batch_create(cvxb_batch **out, int nprob, int n, int m, int device) {
     if (device < 0 || device >= cnt) { set_error("device out of range"); return CVXB_E_ARG; }
     CVXB_CUDA(cudaSetDevice(device));
     cvxb_batch *b = new cvxb_batch();
-    b->device = device; b->B = nprob; b->n = n; b->m = m;
+    b->device = device; b->B = nprob; b->n = n; b->m = m; b->neq = p;
     if (const char *e = getenv("CVXB_OZAKI")) b->i8_mode = (e[0] == '0') ? 0 : (e[0] == '2') ? 2 : 1;
     if (const char *e = getenv("CVXB_OZAKI_IPM")) b->i8_mode = (e[0] == '1') ? 1 : (e[0] == '2') ? 2 : 0;
     b->ldg = ((m + 1) & ~1) > 2 ? ((m + 1) & ~1) : 2;
@@ -441,7 +611,10 @@ int cvxb_batch_create(cvxb_batch **out, int nprob, int n, int m, int device) {
     BCUDA(cudaMalloc(&b->K, B * b->sK * sizeof(double)));
     BCUDA(cudaMalloc(&b->inv, B * b->sInv * sizeof(double)));
     BCUDA(cudaMalloc(&b->panel, B * (size_t)((n + 1) & ~1) * NB * sizeof(double)));
-    BCUDA(cudaMalloc(&b->gemv_ws, B * (size_t)(m > 0 ? m : 1) * gemv_n_chunks(n) * sizeof(double)));
+    {   // gemv_n workspace: rows of G, and with p > 0 also the n rows of Asct
+        const size_t rows = (size_t)std::max(std::max(m, p > 0 ? n : 0), 1);
+        BCUDA(cudaMalloc(&b->gemv_ws, B * rows * gemv_n_chunks(n) * sizeof(double)));
+    }
     // vectors: n-sized: q x rx dx ; m-sized: h s z rz ds dz lmbda lmbdasq d di di2 ws3 bzp
     const size_t nv = 4, mv = 13;
     const size_t me = (size_t)(m > 0 ? m : 1);
@@ -454,6 +627,25 @@ int cvxb_batch_create(cvxb_batch **out, int nprob, int n, int m, int device) {
     b->p.dz = take(me); b->p.lmbda = take(me); b->p.lmbdasq = take(me); b->p.d = take(me);
     b->p.di = take(me); b->p.di2 = take(me); b->p.ws3 = take(me); b->p.bzp = take(me);
     b->p.q = b->q; b->p.h = b->h; b->p.n = n; b->p.m = m;
+    b->p.neq = p; b->p.beq = nullptr; b->p.y = b->p.ry = b->p.dy = b->p.wsing = nullptr;
+    if (p > 0) {
+        b->lda = b->ldkp = (p + 1) & ~1;
+        b->sA = b->lda * n; b->sAs = b->ldk * p; b->sKp = b->ldkp * p;
+        b->sInvp = (long long)2 * ((p + NB - 1) / NB) * NB * NB;
+        BCUDA(cudaMalloc(&b->A, B * b->sA * sizeof(double)));
+        BCUDA(cudaMalloc(&b->Asct, B * b->sAs * sizeof(double)));
+        BCUDA(cudaMalloc(&b->Kp, B * b->sKp * sizeof(double)));
+        BCUDA(cudaMalloc(&b->invp, B * b->sInvp * sizeof(double)));
+        BCUDA(cudaMalloc(&b->veq, B * 5 * (size_t)p * sizeof(double)));
+        BCUDA(cudaMemset(b->veq, 0, B * 5 * (size_t)p * sizeof(double)));
+        BCUDA(cudaMalloc(&b->d_infop, B * sizeof(int)));
+        BCUDA(cudaMalloc(&b->d_nsing, sizeof(int)));
+        double *w = b->veq;
+        b->p.beq = w; b->p.y = w + B * p; b->p.ry = w + 2 * B * p; b->p.dy = w + 3 * B * p; b->p.wsing = w + 4 * B * p;
+    }
+    if (const char *e = getenv("CVXB_BATCH_PHASE_MS")) b->time_phases = e[0] == '1';
+    if (b->time_phases)
+        for (cudaEvent_t &e : b->ph) BCUDA(cudaEventCreate(&e));
     BCUDA(cudaMalloc(&b->sc, B * sizeof(Scal)));
     BCUDA(cudaMemset(b->sc, 0, B * sizeof(Scal)));
     b->p.sc = b->sc;
@@ -474,8 +666,11 @@ void cvxb_batch_destroy(cvxb_batch *b) {
     if (!b) return;
     cudaSetDevice(b->device);
     if (b->st) cudaStreamSynchronize(b->st);
-    double *bufs[] = {b->P, b->G, b->K, b->inv, b->panel, b->gemv_ws, b->vecs};
+    double *bufs[] = {b->P, b->G, b->K, b->inv, b->panel, b->gemv_ws, b->vecs, b->A, b->Asct, b->Kp, b->invp, b->veq};
     for (double *x : bufs) if (x) cudaFree(x);
+    if (b->d_infop) cudaFree(b->d_infop);
+    if (b->d_nsing) cudaFree(b->d_nsing);
+    for (cudaEvent_t e : b->ph) if (e) cudaEventDestroy(e);
     if (b->sc) cudaFree(b->sc);
     if (b->oz_work) cudaFree(b->oz_work);
     if (b->d_info) cudaFree(b->d_info);
@@ -510,6 +705,7 @@ int cvxb_batch_load(cvxb_batch *b, const double *P, const double *q, const doubl
     CVXB_TRY(symmetrize_lower(b->n, b->P, b->ldp, b->B, b->sP, b->st));
     CVXB_CUDA(cudaStreamSynchronize(b->st));
     b->loaded = true;
+    b->eq_loaded = false;        // A and b are loaded after P, q, G, h (cvxb_batch_load_eq)
     for (size_t i = 0; i < B; ++i) b->perm[i] = (int)i;
     b->permuted = false;
     return 0;
@@ -523,6 +719,7 @@ static int swap_slots(cvxb_batch *b, const std::vector<int> &pairs) {
     SwapArgs a;
     a.P = b->P; a.G = b->G; a.vecs = b->vecs; a.sc = b->sc; a.sP = b->sP; a.sG = b->sG;
     a.n = b->n; a.me = b->m > 0 ? b->m : 1; a.Btot = b->B;
+    a.A = b->A; a.veq = b->veq; a.sA = b->sA; a.neq = b->neq;
     k_swap_slots<<<dim3(96, np), 256, 0, b->st>>>(a, b->d_pairs);
     count_launch();
     // `pairs` is pageable host memory: the copy above is staged before cudaMemcpyAsync returns
@@ -546,8 +743,27 @@ static int restore_order(cvxb_batch *b) {
     return 0;
 }
 
+// A: nprob x (p x n column-major, ld p) ; bvec: nprob x p.  After cvxb_batch_load.
+int cvxb_batch_load_eq(cvxb_batch *b, const double *A, const double *bvec, int space) {
+    if (!b) { set_error("batch is NULL"); return CVXB_E_ARG; }
+    if (!b->loaded) { set_error("batch_load_eq: call cvxb_batch_load first"); return CVXB_E_ARG; }
+    if (b->neq == 0) { b->eq_loaded = true; return 0; }
+    if (!A || !bvec) { set_error("batch_load_eq: NULL argument"); return CVXB_E_ARG; }
+    CVXB_CUDA(cudaSetDevice(b->device));
+    CVXB_TRY(restore_order(b));
+    const cudaMemcpyKind kind = (space == CVXB_DEVICE) ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    const size_t B = b->B, n = b->n, p = b->neq;
+    CVXB_CUDA(cudaMemcpy2DAsync(b->A, b->lda * sizeof(double), A, p * sizeof(double), p * sizeof(double), n * B,
+                                kind, b->st));
+    CVXB_CUDA(cudaMemcpyAsync(const_cast<double *>(b->p.beq), bvec, B * p * sizeof(double), kind, b->st));
+    CVXB_CUDA(cudaStreamSynchronize(b->st));
+    b->eq_loaded = true;
+    return 0;
+}
+
 int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, double feastol) {
     if (!b || !b->loaded) { set_error("batch_solve: load the problems first"); return CVXB_E_ARG; }
+    if (b->neq > 0 && !b->eq_loaded) { set_error("batch_solve: load A and b (cvxb_batch_load_eq) first"); return CVXB_E_ARG; }
     CVXB_CUDA(cudaSetDevice(b->device));
     cudaStream_t st = b->st;
     CVXB_TRY(restore_order(b));
@@ -559,10 +775,15 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
     GemvBatch gGt; gGt.batch = B; gGt.sA = b->sG; gGt.sx = m; gGt.sy = n;
     GemvBatch gGn; gGn.batch = B; gGn.sA = b->sG; gGn.sx = n; gGn.sy = m;
     CVXB_CUDA(cudaMemsetAsync(b->sc, 0, (size_t)B * sizeof(Scal), st));
+    b->nsing = 0;
+    if (b->neq > 0) CVXB_CUDA(cudaMemsetAsync(p.wsing, 0, (size_t)B * b->neq * sizeof(double), st));
+    for (double &t : b->phase_ms) t = 0;
+    GemvBatch gAt; gAt.batch = B; gAt.sA = b->sA; gAt.sx = b->neq; gAt.sy = n;
+    GemvBatch gAn; gAn.batch = B; gAn.sA = b->sA; gAn.sx = n; gAn.sy = b->neq;
     CVXB_CUDA(cudaEventRecord(b->e0, st));
     // ---- starting point: W = I ----
     k_init_rhs<<<B, T, 0, st>>>(p); count_launch();
-    CVXB_TRY(batch_factor(b));
+    CVXB_TRY(batch_factor(b, true));
     k_scale_bz<<<B, T, 0, st>>>(p, p.dz); count_launch();
     CVXB_TRY(batch_solve(b));
     k_init_point<<<B, T, 0, st>>>(p); count_launch();
@@ -575,7 +796,11 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
         CVXB_CUDA(cudaStreamSynchronize(st));
         for (int i = 0; i < B; ++i) if (info[i] > 0) { info_fail = i + 1; break; }
         if (info_fail) {
-            set_error("batch_solve: problem %d: Rank([P; G]) < n (singular KKT matrix at the start)", info_fail - 1);
+            if (b->neq > 0)
+                set_error("batch_solve: problem %d: Rank(A) < p or Rank([P; A; G]) < n (singular KKT matrix at the "
+                          "start)", info_fail - 1);
+            else
+                set_error("batch_solve: problem %d: Rank([P; G]) < n (singular KKT matrix at the start)", info_fail - 1);
             return CVXB_E_ARG;
         }
     }
@@ -586,10 +811,13 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
         k_res_begin<<<B, T, 0, st>>>(p); count_launch();
         CVXB_TRY(gemv_t(n, n, b->P, b->ldp, nullptr, p.x, 1.0, 1.0, p.rx, st, gP));
         k_res_dots<<<B, T, 0, st>>>(p); count_launch();
+        if (b->neq > 0) CVXB_TRY(gemv_t(b->neq, n, b->A, b->lda, nullptr, p.y, 1.0, 1.0, p.rx, st, gAt));   // rx += A'y
         if (m > 0) {
             CVXB_TRY(gemv_t(m, n, b->G, b->ldg, nullptr, p.z, 1.0, 1.0, p.rx, st, gGt));
             CVXB_TRY(gemv_n(m, n, b->G, b->ldg, nullptr, p.x, 1.0, 1.0, p.rz, b->gemv_ws, st, gGn));
         }
+        if (b->neq > 0)        // ry := A x - b
+            CVXB_TRY(gemv_n(b->neq, n, b->A, b->lda, nullptr, p.x, 1.0, -1.0, p.ry, b->gemv_ws, st, gAn));
         CVXB_CUDA(cudaMemsetAsync(b->d_ndone, 0, sizeof(int), st));
         k_stats<<<B, T, 0, st>>>(p, it, maxiters, abstol, reltol, feastol, b->d_ndone, b->d_done); count_launch();
         int ndone = 0;
@@ -613,7 +841,7 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
             b->permuted = true;
             B = nb;
             b->Bact = B;
-            gP.batch = gGt.batch = gGn.batch = B;
+            gP.batch = gGt.batch = gGn.batch = gAt.batch = gAn.batch = B;
         }
         k_scaling<<<B, T, 0, st>>>(p, it == 0 ? 1 : 0); count_launch();
         CVXB_TRY(batch_factor(b));
@@ -635,26 +863,30 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
     return 0;
 }
 
+// dst[problem, :len] = src[slot, :len] for every slot (rows of length len, one per problem)
+static int give_rows(cvxb_batch *b, double *dst, const double *src, int len, int space) {
+    const cudaMemcpyKind kind = (space == CVXB_DEVICE) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    const size_t B = b->B;
+    if (!b->permuted) { CVXB_CUDA(cudaMemcpy(dst, src, B * len * sizeof(double), kind)); return 0; }
+    // slot -> problem (identity unless the solve compacted finished problems away)
+    CVXB_CUDA(cudaMemcpy(b->d_perm, b->perm.data(), B * sizeof(int), cudaMemcpyHostToDevice));
+    double *tmp = (space == CVXB_DEVICE) ? dst : nullptr;
+    if (!tmp) CVXB_CUDA(tmp_malloc(&tmp, B * len * sizeof(double)));
+    k_unpermute_rows<<<(unsigned)B, 256, 0, b->st>>>(src, tmp, b->d_perm, len);
+    count_launch();
+    cudaError_t e = cudaStreamSynchronize(b->st);
+    if (e == cudaSuccess && tmp != dst) e = cudaMemcpy(dst, tmp, B * len * sizeof(double), kind);
+    if (tmp != dst) tmp_free(tmp);
+    CVXB_CUDA(e);
+    return 0;
+}
+
 int cvxb_batch_results(cvxb_batch *b, double *x, double *s, double *z, int *status, int *iters,
                        double *pobj, double *dobj, int space) {
     if (!b) { set_error("batch is NULL"); return CVXB_E_ARG; }
     CVXB_CUDA(cudaSetDevice(b->device));
-    const cudaMemcpyKind kind = (space == CVXB_DEVICE) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
     const size_t B = b->B;
-    // slot -> problem (identity unless the solve compacted finished problems away)
-    if (b->permuted) CVXB_CUDA(cudaMemcpy(b->d_perm, b->perm.data(), B * sizeof(int), cudaMemcpyHostToDevice));
-    auto give = [&](double *dst, const double *src, int len) -> int {
-        if (!b->permuted) { CVXB_CUDA(cudaMemcpy(dst, src, B * len * sizeof(double), kind)); return 0; }
-        double *tmp = (space == CVXB_DEVICE) ? dst : nullptr;
-        if (!tmp) CVXB_CUDA(tmp_malloc(&tmp, B * len * sizeof(double)));
-        k_unpermute_rows<<<(unsigned)B, 256, 0, b->st>>>(src, tmp, b->d_perm, len);
-        count_launch();
-        cudaError_t e = cudaStreamSynchronize(b->st);
-        if (e == cudaSuccess && tmp != dst) e = cudaMemcpy(dst, tmp, B * len * sizeof(double), kind);
-        if (tmp != dst) tmp_free(tmp);
-        CVXB_CUDA(e);
-        return 0;
-    };
+    auto give = [&](double *dst, const double *src, int len) { return give_rows(b, dst, src, len, space); };
     if (x) CVXB_TRY(give(x, b->p.x, b->n));
     if (s && b->m) CVXB_TRY(give(s, b->p.s, b->m));
     if (z && b->m) CVXB_TRY(give(z, b->p.z, b->m));
@@ -670,6 +902,29 @@ int cvxb_batch_results(cvxb_batch *b, double *x, double *s, double *z, int *stat
             if (dobj) dobj[i] = sc[slot].dcost;
         }
     }
+    return 0;
+}
+
+int cvxb_batch_results_y(cvxb_batch *b, double *y, int space) {
+    if (!b || !y) { set_error("batch_results_y: NULL argument"); return CVXB_E_ARG; }
+    if (b->neq == 0) return 0;
+    CVXB_CUDA(cudaSetDevice(b->device));
+    return give_rows(b, y, b->p.y, b->neq, space);
+}
+
+int cvxb_batch_singular(cvxb_batch *b, int *flags) {
+    if (!b || !flags) { set_error("batch_singular: NULL argument"); return CVXB_E_ARG; }
+    CVXB_CUDA(cudaSetDevice(b->device));
+    std::vector<Scal> sc(b->B);
+    CVXB_CUDA(cudaMemcpy(sc.data(), b->sc, sc.size() * sizeof(Scal), cudaMemcpyDeviceToHost));
+    for (int slot = 0; slot < b->B; ++slot) flags[b->perm[slot]] = sc[slot].singular;
+    return 0;
+}
+
+int cvxb_batch_phase_ms(cvxb_batch *b, double *ms) {
+    if (!b || !ms) { set_error("batch_phase_ms: NULL argument"); return CVXB_E_ARG; }
+    if (!b->time_phases) { set_error("batch_phase_ms: create the batch with CVXB_BATCH_PHASE_MS=1"); return CVXB_E_ARG; }
+    for (int k = 0; k < 3; ++k) ms[k] = b->phase_ms[k];
     return 0;
 }
 

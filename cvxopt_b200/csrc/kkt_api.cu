@@ -200,8 +200,8 @@ int kkt_unpack_z(cvxb_kkt *k, double *zd) {
 }
 
 int trsm_lower_left(int n, const double *L, long long ldl, const double *inv, double *B, long long ldb, int ncols,
-                    cudaStream_t st) {
-    if (n <= 0 || ncols <= 0) return 0;
+                    cudaStream_t st, int batch, long long sL, long long sInv, long long sB) {
+    if (n <= 0 || ncols <= 0 || batch <= 0) return 0;
     const int nblk = (n + NB - 1) / NB;
     for (int jb = 0; jb < nblk; ++jb) {
         const int j = jb * NB;
@@ -214,6 +214,7 @@ int trsm_lower_left(int n, const double *L, long long ldl, const double *inv, do
             g.X = inv + (long long)jb * NB * NB; g.ldx = NB; g.x_kmajor = false;
             g.Y = Bj; g.ldy = (int)ldb; g.y_kmajor = true;
             g.C = Bj; g.ldc = (int)ldb;
+            g.batch = batch; g.sX = sInv; g.sY = sB; g.sC = sB;
             CVXB_TRY(dmma_gemm(g, st));
         }
         if (mrem > 0) {   // B[j+1:, :] -= L[j+1:, j] X_j
@@ -223,6 +224,7 @@ int trsm_lower_left(int n, const double *L, long long ldl, const double *inv, do
             g.Y = Bj; g.ldy = (int)ldb; g.y_kmajor = true;
             g.D = Bj + wj; g.ldd = (int)ldb; g.C = Bj + wj; g.ldc = (int)ldb;
             g.alpha = -1.0; g.beta = 1.0;
+            g.batch = batch; g.sX = sL; g.sY = sB; g.sD = sB; g.sC = sB;
             CVXB_TRY(dmma_gemm(g, st));
         }
     }

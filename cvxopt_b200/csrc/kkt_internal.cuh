@@ -67,8 +67,9 @@ int xfer_vec(double *dst, const double *src, size_t n, int space, bool to_device
 inline long long kkt_ldk(const cvxb_kkt *k) { long long l = (k->n + 1) & ~1; return l > 2 ? l : 2; }
 // B := L^{-1} B for the n x n Cholesky factor L (lower, ld ldl) with its diagonal-block inverses `inv`
 // (potrf_lower's output); B is n x ncols (ld ldb), updated in place by blocked forward substitution (DMMA GEMMs).
+// Batched (blockIdx.z of every GEMM): problem b uses L + b*sL, inv + b*sInv, B + b*sB.
 int trsm_lower_left(int n, const double *L, long long ldl, const double *inv, double *B, long long ldb, int ncols,
-                    cudaStream_t st);
+                    cudaStream_t st, int batch = 1, long long sL = 0, long long sInv = 0, long long sB = 0);
 int kkt_pack_bz(cvxb_kkt *k, const double *zd);      // k->bzp := pack(W^{-T} bz)
 int kkt_unpack_z(cvxb_kkt *k, double *zd);           // z := unpack(k->bzp)
 // route-specific factor / solve (kkt_qr.cu, kkt_ldl.cu)

@@ -205,17 +205,33 @@ int cvxb_gemm(int transa, int transb, int m, int n, int k, double alpha, const d
 
 /* ---- batch of independent dense QPs (BASELINE config 4): one problem per
  * CTA-group, lock-step primal-dual IPM fully on device (oracle: a Python loop
- * over solvers.qp).  Problems are  min 1/2 x'P x + q'x  s.t.  G x <= h. */
+ * over solvers.qp).  Problems are  min 1/2 x'P x + q'x  s.t.  G x <= h, A x = b,
+ * A with p rows (0 <= p <= n; p > 0 needs m > 0).  With p > 0 every problem
+ * follows coneqp with kktsolver='chol2' (solvers.qp(P, q, G, h, A, b)).
+ * cvxb_batch_create is cvxb_batch_create_eq with p = 0. */
 int cvxb_batch_create(cvxb_batch **out, int nprob, int n, int m, int device);
+int cvxb_batch_create_eq(cvxb_batch **out, int nprob, int n, int m, int p, int device);
 void cvxb_batch_destroy(cvxb_batch *b);
 /* P: nprob x (n x n, ld n); q: nprob x n; G: nprob x (m x n column-major, ld m); h: nprob x m */
 int cvxb_batch_load(cvxb_batch *b, const double *P, const double *q, const double *G,
                     const double *h, int space);
+/* A: nprob x (p x n column-major, ld p); bvec: nprob x p.  Required after every
+ * cvxb_batch_load when p > 0 (a no-op when p = 0). */
+int cvxb_batch_load_eq(cvxb_batch *b, const double *A, const double *bvec, int space);
 int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, double feastol);
 /* status: 1 optimal, 2 maximum iterations reached, 3 singular KKT matrix ('unknown' in the
  * reference for 2 and 3).  x/s/z may be device pointers (space), scalars go to host memory. */
 int cvxb_batch_results(cvxb_batch *b, double *x, double *s, double *z, int *status,
                        int *iters, double *pobj, double *dobj, int space);
+/* y: nprob x p multipliers of A x = b (host or device memory, space) */
+int cvxb_batch_results_y(cvxb_batch *b, double *y, int space);
+/* flags (host, nprob): 1 where S = P + G'W^-1 W^-T G was singular at the starting point,
+ * so that S + A'A was factored instead (the reference's kkt_chol2 'singular' branch) */
+int cvxb_batch_singular(cvxb_batch *b, int *flags);
+/* ms[3]: time of the last solve's factorisations by phase: S (SYRK + Cholesky),
+ * L^{-1} A' (TRSM), A S^{-1} A' (SYRK + Cholesky).  Only for a batch created with
+ * CVXB_BATCH_PHASE_MS=1, which synchronises after every phase. */
+int cvxb_batch_phase_ms(cvxb_batch *b, double *ms);
 /* CUDA-event time of the last cvxb_batch_solve and the number of lock-step iterations run */
 int cvxb_batch_stats(cvxb_batch *b, double *solve_ms, int *iterations);
 /* kernel of the factorisations' SYRK in the last solve: 1 fp64 DMMA, 2 int8 slices (as cvxb_kkt_syrk_path) */

@@ -89,6 +89,10 @@ _SIGS = {
                             C.c_int, C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_int, C.c_int]),
     "cvxb_batch_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int]),
     "cvxb_batch_create_eq": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "cvxb_batch_create_cones": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                          C.c_int, C.c_int]),
+    "cvxb_batch_solve_ref": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int]),
+    "cvxb_batch_phase_ms_cones": (C.c_int, [C.c_void_p, c_double_p]),
     "cvxb_batch_destroy": (None, [C.c_void_p]),
     "cvxb_batch_load_eq": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "cvxb_batch_results_y": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),

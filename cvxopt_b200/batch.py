@@ -1,6 +1,11 @@
 """Batch of independent dense QPs solved in lock-step on the device (BASELINE config 4).
 
-    minimize 1/2 x'P x + q'x   subject to   G x <= h,  A x = b     (one 'l' cone of m rows, p rows of A)
+    minimize 1/2 x'P x + q'x   subject to   G x + s = h,  s in C,  A x = b     (p rows of A)
+
+C is one 'l' cone of m rows by default.  With dims = {'l': ml, 'q': [q_1 .. q_K], 's': []} it is ml linear rows
+followed by K second-order cones, the same for every problem of the batch; each problem is then solved as
+coneqp(P, q, G, h, dims[, A, b]) with the reference's default options (kktsolver='chol', one step of iterative
+refinement), which the batch replaces by the equivalent kkt_chol2 elimination.
 
 The per-problem algorithm is coneprog.coneqp restricted to dims={'l': m} (reference
 src/python/coneprog.py:1998-2547) — same start, stopping rule, Mehrotra steps — so every
@@ -57,13 +62,45 @@ def _stack_eq(A, b, B, n):
     return np.ascontiguousarray(np.transpose(A, (0, 2, 1))), b, p
 
 
+def _check_dims(dims, m):
+    """-> (ml, [q_1 .. q_K]) of a cone dimension dict for G with m rows; dims=None is {'l': m, 'q': [], 's': []}.
+    Raises TypeError for malformed dims, 's' cones (not supported by the batch) or sizes that do not add up to m."""
+    if dims is None:
+        return int(m), []
+    if not isinstance(dims, dict):
+        raise TypeError("dims must be a dict with keys 'l', 'q', 's'")
+    ml, ql, sl = dims.get("l", 0), list(dims.get("q", [])), list(dims.get("s", []))
+    ints = (int, np.integer)
+    if not isinstance(ml, ints) or isinstance(ml, bool) or ml < 0:
+        raise TypeError("dims['l'] must be a nonnegative integer")
+    if any(not isinstance(k, ints) or isinstance(k, bool) or k < 1 for k in ql):
+        raise TypeError("dims['q'] must be a list of positive integers")
+    if sl:
+        raise TypeError("the batch solver has no 's' cones: dims['s'] must be empty")
+    if int(ml) + sum(int(k) for k in ql) != m:
+        raise TypeError("dims: l + sum(q) = %d, but G and h have %d rows" % (int(ml) + sum(int(k) for k in ql), m))
+    return int(ml), [int(k) for k in ql]
+
+
+def _refinement(options):
+    """options['refinement'] as the library takes it: -1 for the reference's default rule"""
+    r = options.get("refinement")
+    if r is None:
+        return -1
+    if not isinstance(r, (int, np.integer)) or isinstance(r, bool) or r < 0:
+        raise ValueError("options['refinement'] must be a nonnegative integer")
+    return int(r)
+
+
 class QPBatch:
-    def __init__(self, nprob, n, m, device=0, p=0):
+    def __init__(self, nprob, n, m, device=0, p=0, dims=None):
         self._lib = _lib.load()
         self._h = C.c_void_p()
         self.B, self.n, self.m, self.p = int(nprob), int(n), int(m), int(p)
-        _lib.check(self._lib.cvxb_batch_create_eq(C.byref(self._h), self.B, self.n, self.m, self.p, device),
-                   "batch")
+        self.ml, self.qdims = _check_dims(dims, self.m)
+        qarr = (C.c_int * max(1, len(self.qdims)))(*self.qdims)
+        _lib.check(self._lib.cvxb_batch_create_cones(C.byref(self._h), self.B, self.n, self.ml, len(self.qdims),
+                                                     qarr, self.p, device), "batch")
 
     def load(self, P, q, G, h, A=None, b=None):
         Pcm, q, Gcm, h, B, n, m = _stack(P, q, G, h)
@@ -86,10 +123,11 @@ class QPBatch:
         _lib.check(self._lib.cvxb_batch_load_eq(self._h, A, b, space), "batch_load_eq")
 
     def solve(self, **options):
+        """options as coneqp's: maxiters, abstol, reltol, feastol, refinement (default: 1 with 'q' cones, else 0)"""
         o = dict(DEFAULTS)
         o.update(options)
-        rc = self._lib.cvxb_batch_solve(self._h, int(o["maxiters"]), float(o["abstol"]),
-                                        float(o["reltol"]), float(o["feastol"]))
+        rc = self._lib.cvxb_batch_solve_ref(self._h, int(o["maxiters"]), float(o["abstol"]),
+                                            float(o["reltol"]), float(o["feastol"]), _refinement(o))
         if rc == _lib.E_ARG and "Rank(" in _lib.last_error():
             raise ValueError(_lib.last_error())       # coneprog.py:2065-2067
         _lib.check(rc, "batch_solve")
@@ -121,7 +159,12 @@ class QPBatch:
         """factorisation time of the last solve by phase (batch created with CVXB_BATCH_PHASE_MS=1)"""
         ms = (C.c_double * 3)()
         _lib.check(self._lib.cvxb_batch_phase_ms(self._h, ms), "batch_phase_ms")
-        return {"S_syrk_potrf_ms": ms[0], "trsm_ms": ms[1], "Kp_syrk_potrf_ms": ms[2]}
+        out = {"S_syrk_potrf_ms": ms[0], "trsm_ms": ms[1], "Kp_syrk_potrf_ms": ms[2]}
+        if self.qdims:
+            mq = (C.c_double * 2)()
+            _lib.check(self._lib.cvxb_batch_phase_ms_cones(self._h, mq), "batch_phase_ms_cones")
+            out.update({"Gs_q_scale_ms": mq[0], "Gs_q_gemm_ms": mq[1]})       # both inside S_syrk_potrf_ms
+        return out
 
     def stats(self):
         ms, it = C.c_double(), C.c_int()
@@ -160,7 +203,7 @@ class QPBatchGroup:
     as ITS slowest problem is done.  Interleaved slices (problem i -> sub-batch i mod nsub) spread hard and easy
     problems evenly."""
 
-    def __init__(self, nprob, n, m, device=0, nsub=None, p=0):
+    def __init__(self, nprob, n, m, device=0, nsub=None, p=0, dims=None):
         if nsub is None:
             # measured on B200 (profiles/r02h_batch_nsub.txt, n=512 m=1024): 512 problems 148 -> 142 ms with 2
             # sub-batches; 64 problems 25.0 -> 21.3 ms with 8
@@ -169,7 +212,8 @@ class QPBatchGroup:
         self.nsub = max(1, min(int(nsub), nprob))
         self.B, self.n, self.m, self.p = int(nprob), int(n), int(m), int(p)
         self.idx = [np.arange(r, self.B, self.nsub) for r in range(self.nsub)]
-        self.parts = [QPBatch(len(ix), n, m, device, p) for ix in self.idx]
+        _check_dims(dims, self.m)
+        self.parts = [QPBatch(len(ix), n, m, device, p, dims) for ix in self.idx]
 
     def load_ptr_sliced(self, loader):
         """loader(part_index, indices, QPBatch) loads one sub-batch (device-resident callers)"""
@@ -235,14 +279,21 @@ class QPBatchGroup:
             b.close()
 
 
-def qp_batch(P, q, G, h, A=None, b=None, device=0, nsub=None, **options):
+def qp_batch(P, q, G, h, A=None, b=None, device=0, nsub=None, dims=None, **options):
     """Solve B independent dense QPs on one GPU.  P (B,n,n), q (B,n), G (B,m,n), h (B,m), and optionally
     equality constraints A (B,p,n), b (B,p) as in solvers.qp(P, q, G, h, A, b).
+    dims: the cone of G x + s = h, {'l': ml, 'q': [q_1 .. q_K], 's': []}, shared by all problems (default: 'l' only);
+    s and z are returned in its order, 'l' rows then the cones.  Options: maxiters, abstol, reltol, feastol and
+    refinement, as coneqp's.
     nsub: number of concurrently solved sub-batches (QPBatchGroup); default 4 (1 for tiny batches)."""
     P = np.asarray(P)
     G = np.asarray(G)
+    if G.ndim != 3:
+        raise TypeError("G must have shape (B, m, n)")
+    _check_dims(dims, G.shape[1])
+    _refinement(options)
     p = 0 if A is None else np.asarray(A).shape[1]
-    grp = QPBatchGroup(P.shape[0], P.shape[1], G.shape[1], device, nsub, p)
+    grp = QPBatchGroup(P.shape[0], P.shape[1], G.shape[1], device, nsub, p, dims)
     try:
         grp.load(P, q, G, h, A, b)
         import time
@@ -292,11 +343,12 @@ def _p2p(ops):
 
 
 def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interleaved", timings=None,
-                         nsub=None, A=None, b=None, **options):
+                         nsub=None, A=None, b=None, dims=None, **options):
     """Rank 0 passes the full batch (other ranks pass None); every rank returns its shard's results and
     rank 0 additionally gets the gathered batch, in the original problem order, under key 'all'.
     Equality constraints A (B,p,n), b (B,p) are optional (rank 0 only); `solver` (a stand-in for the
-    device solver) is then called as solver(P, q, G, h, A, b).
+    device solver) is then called as solver(P, q, G, h, A, b).  dims (rank 0's) is the cone of every problem, as
+    in qp_batch; with 'q' cones the stand-in is called with dims= as well.
 
     `timings` (dict, optional) receives scatter_ms / solve_ms / gather_ms of this rank, measured with
     device events on the current stream (wall clock on CPU)."""
@@ -332,17 +384,26 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
                 self.t[name] = (time.perf_counter() - e0) * 1e3
     clk = _Clock()
 
-    meta = torch.zeros(4, dtype=torch.int64, device=dev)
+    meta = torch.zeros(6, dtype=torch.int64, device=dev)
     full = None
+    qlist = []
     if rank == 0:
         # the batch in the layout QPBatch loads: column-major n x n / m x n / p x n per problem
         Pcm, qh, Gcm, hh, Btot, n, m = _stack(P, q, G, h)
         Acm, bh, p = _stack_eq(A, b, Btot, n)
-        meta = torch.tensor([Btot, n, m, p], dtype=torch.int64, device=dev)
+        ml, qlist = _check_dims(dims, m)
+        _refinement(options)
+        meta = torch.tensor([Btot, n, m, p, ml, len(qlist)], dtype=torch.int64, device=dev)
         full = [torch.from_numpy(a).to(dev) for a in ((Pcm, qh, Gcm, hh) + ((Acm, bh) if p else ()))]  # one H2D
     if world > 1:
         dist.broadcast(meta, 0, group=group)
-    Btot, n, m, p = (int(v) for v in meta.tolist())
+    Btot, n, m, p, ml, nq = (int(v) for v in meta.tolist())
+    if nq and world > 1:                    # the cone sizes: one more broadcast, only with 'q' cones
+        qt = torch.tensor(qlist, dtype=torch.int64, device=dev) if rank == 0 else \
+            torch.zeros(nq, dtype=torch.int64, device=dev)
+        dist.broadcast(qt, 0, group=group)
+        qlist = [int(v) for v in qt.tolist()]
+    dims = {"l": ml, "q": qlist, "s": []}
     owners = shard_indices(Btot, world, sharding)
     mine = owners[rank]
     k = len(mine)
@@ -351,7 +412,7 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
     # ---- setup (not data path): this rank's batch object = its device allocations ----
     local_dev = torch.cuda.current_device() if on_gpu else 0
     clk.start("setup_ms")
-    bobj = QPBatchGroup(k, n, m, local_dev, nsub, p) if (solver is None and k) else None
+    bobj = QPBatchGroup(k, n, m, local_dev, nsub, p, dims) if (solver is None and k) else None
     clk.stop()
 
     # ---- scatter ----
@@ -385,7 +446,7 @@ def qp_batch_distributed(P, q, G, h, solver=None, group=None, sharding="interlea
         args = [np.transpose(sh[0], (0, 2, 1)), sh[1], np.transpose(sh[2], (0, 2, 1)), sh[3]]
         if p:
             args += [np.transpose(sh[4], (0, 2, 1)), sh[5]]
-        res = solver(*args) if k else None
+        res = (solver(*args, dims=dims) if nq else solver(*args)) if k else None
 
         def rows(key, d):
             if not k or not d:

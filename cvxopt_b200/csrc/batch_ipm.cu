@@ -16,6 +16,13 @@
 // misc.kkt_chol2 (misc.py:1352-1567): S = P + G' D^-2 G = L L', Asct = L^{-1} A', Kp = Asct' Asct = Lp Lp'.
 // A problem whose S is singular at the starting point (W = I) factors S + A'A from then on (misc.py:1421-1461);
 // per problem, through a 0/1 weight vector of length p (`wsing`) applied inside the batched GEMM / GEMV.
+//
+// Second-order cones: the inequality rows may be dims = {'l': ml, 'q': [q_1 .. q_K]} (the same for every problem), and
+// the algorithm is then coneqp with that dims and its default options (:1805-1809, :1862-1865): one step of iterative
+// refinement per Newton solve (f4, :2330-2347; any count through options['refinement'], for 'l'-only batches too) and
+// the same kkt_chol2 elimination, with the cones' rows scaled explicitly (Gs_q = W^{-T} G_q) and added to S by a second
+// batched GEMM.  The cone kernels walk a problem's cones with one thread, a warp or the CTA per cone (GThread / GWarp /
+// GBlock below), chosen at create from the cone sizes.
 #include "kkt_internal.cuh"
 #include <algorithm>
 #include <cstdlib>
@@ -60,6 +67,205 @@ __device__ __forceinline__ double block_min(double v, double *sh) {
     __syncthreads();
     return sh[0];
 }
+__device__ __forceinline__ double block_max(double v, double *sh) { return -block_min(-v, sh); }
+
+// ---- 'q' cones: the threads that work on one cone ("group") ----
+// Every problem has the same cones; a CTA (one problem) walks them with groups of 1 thread (tiny cones), a warp
+// (many cones) or the whole CTA (a few large cones).  Group g takes cones g, g + ngroups, ...; element i of a cone
+// belongs to the group's thread i mod size, and element 0 to rank 0.  sum() reduces over the group and returns the
+// total to every member; it orders the members' earlier global writes before their later reads.
+struct GThread {
+    __device__ int rank() const { return 0; }
+    __device__ int size() const { return 1; }
+    __device__ int gid() const { return threadIdx.x; }
+    __device__ int ngroups() const { return blockDim.x; }
+    __device__ double sum(double v, double *) const { return v; }
+    __device__ void sync() const {}
+};
+struct GWarp {
+    __device__ int rank() const { return threadIdx.x & 31; }
+    __device__ int size() const { return 32; }
+    __device__ int gid() const { return threadIdx.x >> 5; }
+    __device__ int ngroups() const { return blockDim.x >> 5; }
+    __device__ double sum(double v, double *) const { __syncwarp(); v = warp_sum(v); __syncwarp(); return v; }
+    __device__ void sync() const { __syncwarp(); }
+};
+struct GBlock {
+    __device__ int rank() const { return threadIdx.x; }
+    __device__ int size() const { return blockDim.x; }
+    __device__ int gid() const { return 0; }
+    __device__ int ngroups() const { return 1; }
+    __device__ double sum(double v, double *sh) const { return block_sum(v, sh); }
+    __device__ void sync() const { __syncthreads(); }
+};
+
+// Per-cone formulas of the reference's cone algebra (misc_solvers.c / misc.py, cited at each helper), in the same
+// arithmetic as the single-problem kernels of cone_vec.cu, nt_scaling.cu and cone.cu.  x, y, ... point at the cone's
+// first element; mq is its size.  Every helper ends with the group synchronised.
+
+// max_step of one cone: ||x1|| - x0  (misc_solvers.c:1083-1093)
+template <class Gp>
+__device__ double q_max_step(const Gp &g, const double *x, int mq, double *sh) {
+    double n2 = 0;
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) n2 += x[i] * x[i];
+    n2 = g.sum(n2, sh);
+    return sqrt(n2) - x[0];
+}
+// x := y o\ x  (sinv, misc_solvers.c:813-850)
+template <class Gp>
+__device__ void q_sinv(const Gp &g, double *x, const double *y, int mq, double *sh) {
+    double n2 = 0, d = 0;
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) { n2 += y[i] * y[i]; d += x[i] * y[i]; }
+    const double y0 = y[0], cx = x[0];
+    n2 = g.sum(n2, sh); d = g.sum(d, sh);
+    const double nrm = sqrt(n2);
+    const double a = (y0 + nrm) * (y0 - nrm);
+    const double al1 = a / y0, al2 = d / y0 - cx, ia = 1.0 / a;
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) x[i] = (x[i] * al1 + al2 * y[i]) * ia;
+    if (g.rank() == 0) x[0] = (cx * y0 - d) * ia;
+    g.sync();
+}
+// x := y o x  (sprod, misc_solvers.c:680-700; the same with diag = 'D')
+template <class Gp>
+__device__ void q_sprod(const Gp &g, double *x, const double *y, int mq, double *sh) {
+    double d = 0;
+    for (int i = g.rank(); i < mq; i += g.size()) d += y[i] * x[i];
+    const double y0 = y[0], x0 = x[0];
+    d = g.sum(d, sh);
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) x[i] = y0 * x[i] + x0 * y[i];
+    if (g.rank() == 0) x[0] = d;
+    g.sync();
+}
+// x := W x = beta (2 v v' - J) x,  or  x := W^{-1} x = (1/beta) (2 J v v' J - J) x  (scale, misc_solvers.c:156-183)
+template <class Gp>
+__device__ void q_scale(const Gp &g, double *x, const double *v, double beta, int mq, bool inverse, double *sh) {
+    double w = 0;
+    for (int i = g.rank(); i < mq; i += g.size()) {
+        double xi = x[i];
+        if (inverse && i == 0) xi = -xi;
+        w += v[i] * xi;
+    }
+    w = g.sum(w, sh);
+    const double tw = 2.0 * w, bb = inverse ? 1.0 / beta : beta;
+    for (int i = g.rank(); i < mq; i += g.size()) {
+        double xi = x[i];
+        if (!inverse && i == 0) xi = -xi;
+        double yi = xi + v[i] * tw;
+        if (inverse && i == 0) yi = -yi;
+        x[i] = yi * bb;
+    }
+    g.sync();
+}
+// x := H(lambda^{1/2}) x or its inverse  (scale2, misc_solvers.c:296-335)
+template <class Gp>
+__device__ void q_scale2(const Gp &g, const double *lm, double *x, int mq, bool inverse, double *sh) {
+    double n2 = 0, dot = 0;
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) { n2 += lm[i] * lm[i]; dot += lm[i] * x[i]; }
+    const double l0 = lm[0], x0 = x[0];
+    n2 = g.sum(n2, sh); dot = g.sum(dot, sh);
+    const double nrm = sqrt(n2);
+    const double a = sqrt(l0 + nrm) * sqrt(l0 - nrm);
+    const double lx = inverse ? (l0 * x0 + dot) / a : (l0 * x0 - dot) / a;
+    double c = (x0 + lx) / (l0 / a + 1.0) / a;
+    if (!inverse) c = -c;
+    const double sc = inverse ? a : 1.0 / a;
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) x[i] = (x[i] + c * lm[i]) * sc;
+    if (g.rank() == 0) x[0] = lx * sc;
+    g.sync();
+}
+// out := lambda o lambda  (ssqr, misc.py:957-962)
+template <class Gp>
+__device__ void q_ssqr(const Gp &g, double *out, const double *lm, int mq, double *sh) {
+    double n2 = 0;
+    for (int i = g.rank(); i < mq; i += g.size()) n2 += lm[i] * lm[i];
+    n2 = g.sum(n2, sh);
+    const double l0 = lm[0];
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) out[i] = 2.0 * l0 * lm[i];
+    if (g.rank() == 0) out[0] = n2;
+    g.sync();
+}
+// sqrt(x' J x) as misc.jnrm2 evaluates it (misc.py:848-856)
+template <class Gp>
+__device__ double q_jnrm2(const Gp &g, const double *x, int mq, double *sh) {
+    double t = 0;
+    for (int i = 1 + g.rank(); i < mq; i += g.size()) t += x[i] * x[i];
+    const double x0 = x[0];
+    const double a = sqrt(g.sum(t, sh));
+    return sqrt(x0 - a) * sqrt(x0 + a);
+}
+// Nesterov-Todd scaling of one cone from s, z: v, beta, lambda  (compute_scaling, misc.py:311-354)
+template <class Gp>
+__device__ void q_compute_scaling(const Gp &g, const double *sk, const double *zk, double *v, double *beta,
+                                  double *lk, int mq, double *sh) {
+    const double aa = q_jnrm2(g, sk, mq, sh), bb = q_jnrm2(g, zk, mq, sh);
+    double t = 0;
+    for (int i = g.rank(); i < mq; i += g.size()) t += sk[i] * zk[i];
+    const double dot = g.sum(t, sh);
+    const double cc = sqrt((dot / aa / bb + 1.0) / 2.0);
+    const double s0 = sk[0], z0 = zk[0];
+    const double v0 = ((s0 / aa) + (z0 / bb)) / 2.0 / cc + 1.0;
+    const double sc = 1.0 / sqrt(2.0 * v0);
+    const double dd = 2.0 * cc + s0 / aa + z0 / bb;
+    const double c1 = (cc + z0 / bb) / dd / aa, c2 = (cc + s0 / aa) / dd / bb, sab = sqrt(aa * bb);
+    for (int i = g.rank(); i < mq; i += g.size()) {
+        if (i == 0) {
+            v[0] = v0 * sc;
+            lk[0] = cc * sab;
+        } else {
+            v[i] = ((sk[i] / aa - zk[i] / bb) / 2.0 / cc) * sc;
+            lk[i] = (c1 * sk[i] + c2 * zk[i]) * sab;
+        }
+    }
+    if (g.rank() == 0) *beta = sqrt(aa / bb);
+    g.sync();
+}
+// scaling update of one cone; sk, zk hold the new iterates in the current scaling and are normalised in place
+// (update_scaling, misc.py:504-573)
+template <class Gp>
+__device__ void q_update_scaling(const Gp &g, double *sk, double *zk, double *v, double *beta, double *lk, int mq,
+                                 double *sh) {
+    const double aa = q_jnrm2(g, sk, mq, sh);
+    for (int i = g.rank(); i < mq; i += g.size()) sk[i] *= 1.0 / aa;
+    g.sync();
+    const double bb = q_jnrm2(g, zk, mq, sh);
+    for (int i = g.rank(); i < mq; i += g.size()) zk[i] *= 1.0 / bb;
+    g.sync();
+    double t1 = 0, t2 = 0, t3 = 0;
+    for (int i = g.rank(); i < mq; i += g.size()) {
+        t1 += sk[i] * zk[i];
+        t2 += v[i] * sk[i];
+        t3 += (i == 0 ? v[i] * zk[i] : -v[i] * zk[i]);     // jdot: v' J z
+    }
+    const double s0 = sk[0], z0 = zk[0], vk0 = v[0];
+    const double dot = g.sum(t1, sh), vs = g.sum(t2, sh), vz = g.sum(t3, sh);
+    const double cc = sqrt((1.0 + dot) / 2.0);
+    const double vq = (vs + vz) / 2.0 / cc, vu = vs - vz;
+    const double wk0 = 2.0 * vk0 * vq - (s0 + z0) / 2.0 / cc;
+    const double dd = (vk0 * vu - s0 / 2.0 + z0 / 2.0) / (wk0 + 1.0);
+    const double sab = sqrt(aa * bb);
+    const double vn0 = 2.0 * vq * vk0 - s0 / 2.0 / cc - 0.5 / cc * z0 + 1.0;
+    const double sc = 1.0 / sqrt(2.0 * vn0);
+    for (int i = g.rank(); i < mq; i += g.size()) {
+        const double vi = v[i], si = sk[i], zi = zk[i];
+        if (i == 0) {
+            lk[0] = cc * sab;
+            v[0] = vn0 * sc;
+        } else {
+            lk[i] = (vi * (2.0 * (-dd * vq + 0.5 * vu)) + 0.5 * (1.0 - dd / cc) * si + 0.5 * (1.0 + dd / cc) * zi) * sab;
+            v[i] = (2.0 * vq * vi + 0.5 / cc * si - 0.5 / cc * zi) * sc;
+        }
+    }
+    if (g.rank() == 0) *beta *= sqrt(aa / bb);
+    g.sync();
+}
+
+// the cone table: sizes and offsets (within the 'q' rows) of the K cones, the same for every problem
+struct QCones {
+    int ml, nq, sumq;               // 'l' rows, number of 'q' cones, their total size
+    const int *dim, *off;           // device arrays of length nq
+    const double *e;                // sumq: 1 at the first row of every cone, else 0 (the identity of the cone)
+    double *vb;                     // per problem (stride sumq + nq): v of every cone, then beta of every cone
+};
 
 struct Ptrs {
     int n, m, neq;                  // neq: rows of A (p)
@@ -67,7 +273,18 @@ struct Ptrs {
     double *x, *s, *z, *rx, *rz, *dx, *ds, *dz, *lmbda, *lmbdasq, *d, *di, *di2, *ws3, *bzp;
     double *y, *ry, *dy, *wsing;    // p-vectors (wsing: 1 where S + A'A is factored, else 0)
     Scal *sc;
+    QCones c;
+    // iterative refinement (allocated by the first solve that asks for it): the right-hand side of the Newton
+    // system (wx wy wz ws), the correction's right-hand side / solution (x2 y2 z2 s2), W^{-1} uz (t3)
+    double *wx, *wy, *wz, *ws, *x2, *y2, *z2, *s2, *t3;
 };
+// cone k of problem b:  rows  om + ml + off[k]  of an m-vector;  v at vb + b (sumq + nq) + off[k]
+#define Q_CONE(k)                                                          \
+    const int mq = p.c.dim[k];                                             \
+    const long long oq = om + p.c.ml + p.c.off[k];                         \
+    double *vq_ = p.c.vb + (long long)b * (p.c.sumq + p.c.nq) + p.c.off[k]; \
+    double *betaq_ = p.c.vb + (long long)b * (p.c.sumq + p.c.nq) + p.c.sumq + k;
+#define Q_LOOP(g) for (int k = (g).gid(); k < p.c.nq; k += (g).ngroups())
 #define PB_SETUP                                                  \
     const int b = blockIdx.x, tid = threadIdx.x, nt = blockDim.x; \
     const long long on = (long long)b * p.n, om = (long long)b * p.m; \
@@ -93,6 +310,11 @@ __global__ void k_init_rhs(Ptrs p) {
         for (int i = tid; i < p.neq; i += nt) { double v = p.beq[op + i]; p.dy[op + i] = v; nb += v * v; }
         nb = block_sum(nb, sh);
     }
+    if (p.c.nq > 0) {                                   // W = I: v = e, beta = 1 (:2058-2060)
+        double *vb = p.c.vb + (long long)b * (p.c.sumq + p.c.nq);
+        for (int i = tid; i < p.c.sumq; i += nt) vb[i] = p.c.e[i];
+        for (int k = tid; k < p.c.nq; k += nt) vb[p.c.sumq + k] = 1.0;
+    }
     if (tid == 0) {
         S.resx0 = fmax(1.0, sqrt(nq));                  // :1998
         S.resy0 = fmax(1.0, sqrt(nb));                  // :1999
@@ -107,8 +329,10 @@ __global__ void k_scale_bz(Ptrs p, const double *bz) {
     for (int i = tid; i < p.m; i += nt) p.bzp[om + i] = p.di[om + i] * bz[om + i];
 }
 // starting point, part 2: x = dx, z = dz (solution), s = -z, shifts (:2083-2106), gap (:2165)
+template <class Gp>
 __global__ void k_init_point(Ptrs p) {
     PB_SETUP
+    const int ml = p.c.ml;
     double ns = 0, mins = INFINITY;
     for (int i = tid; i < p.n; i += nt) p.x[on + i] = p.dx[on + i];
     const long long op = (long long)b * p.neq;
@@ -117,21 +341,33 @@ __global__ void k_init_point(Ptrs p) {
         double zv = p.bzp[om + i];      // solve leaves W*uz in bzp
         p.z[om + i] = zv;
         p.s[om + i] = -zv;
-        ns += zv * zv;
-        mins = fmin(mins, -zv);
+        ns += zv * zv;                  // snrm2 == 2-norm for 'l' and 'q'
+        if (i < ml) mins = fmin(mins, -zv);
     }
     ns = sqrt(block_sum(ns, sh));
     mins = block_min(mins, sh);
-    const double ts = -mins;                             // max_step(s) = -min(s) for 'l'
+    double ts = -mins;                                   // max_step(s) = -min(s) for 'l'
     double minz = INFINITY;
-    for (int i = tid; i < p.m; i += nt) minz = fmin(minz, p.z[om + i]);
+    for (int i = tid; i < ml; i += nt) minz = fmin(minz, p.z[om + i]);
     minz = block_min(minz, sh);
-    const double tz = -minz;
+    double tz = -minz;
+    if (p.c.nq > 0) {                                    // and max over the cones of ||x1|| - x0
+        const Gp g;
+        double tsq = -INFINITY, tzq = -INFINITY;
+        Q_LOOP(g) {
+            Q_CONE(k) (void)vq_; (void)betaq_;
+            tsq = fmax(tsq, q_max_step(g, p.s + oq, mq, sh));
+            tzq = fmax(tzq, q_max_step(g, p.z + oq, mq, sh));
+        }
+        ts = fmax(ts, block_max(tsq, sh));
+        tz = fmax(tz, block_max(tzq, sh));
+    }
     const double as = (ts >= -1e-8 * fmax(ns, 1.0)) ? 1.0 + ts : 0.0;
     const double az = (tz >= -1e-8 * fmax(ns, 1.0)) ? 1.0 + tz : 0.0;   // nrmz == nrms here
     double gap = 0;
     for (int i = tid; i < p.m; i += nt) {
-        double sv = p.s[om + i] + as, zv = p.z[om + i] + az;
+        const double e = i < ml ? 1.0 : p.c.e[i - ml];  // every 'l' row, the first row of every cone
+        double sv = p.s[om + i] + as * e, zv = p.z[om + i] + az * e;
         p.s[om + i] = sv; p.z[om + i] = zv;
         gap += sv * zv;
     }
@@ -195,20 +431,22 @@ __global__ void k_stats(Ptrs p, int iter, int maxiters, double abstol, double re
 // ---- compaction of finished problems ----
 // The lock-step loop launches every batched kernel over the first `Bact` slots.  When problems finish, each finished
 // slot below the new active count trades places with an active slot from the tail: everything a problem owns between
-// iterations (P, G, A, its 17 + 5 vectors, its scalars; K / inv / info / Asct / Kp are rebuilt every iteration) is swapped,
+// iterations (P, G, A, its 17 + 5 vectors, v and beta of its cones, its scalars; K / inv / info / Asct / Kp / Gs_q and
+// the refinement vectors are rebuilt every iteration) is swapped,
 // so the active
 // problems stay a contiguous prefix and finished ones keep their final iterates in the tail.  ~6.3 MB per swap at
 // n=512, m=1024 (p = 0), at most one swap per problem per solve.
 struct SwapArgs {
-    double *P, *G, *vecs, *A, *veq; Scal *sc;
+    double *P, *G, *vecs, *A, *veq, *vb; Scal *sc;
     long long sP, sG, sA;
-    int n, me, neq, Btot;
+    int n, me, neq, nvb, Btot;      // nvb: v and beta of the 'q' cones (sumq + nq, 0 without cones)
 };
 __global__ void k_swap_slots(SwapArgs a, const int *pairs) {
     const int i = pairs[2 * blockIdx.y], j = pairs[2 * blockIdx.y + 1];
     const long long eP = a.sP, eG = a.sG, eN = 4LL * a.n, eM = 13LL * a.me, eS = (long long)(sizeof(Scal) / sizeof(double));
     const long long eA = a.sA, eQ = 5LL * a.neq;          // both 0 without equality constraints
-    const long long total = eP + eG + eN + eM + eS + eA + eQ;
+    const long long eV = a.nvb;
+    const long long total = eP + eG + eN + eM + eS + eA + eQ + eV;
     for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
         double *x, *y;
         long long r = e;
@@ -226,8 +464,10 @@ __global__ void k_swap_slots(SwapArgs a, const int *pairs) {
             x = reinterpret_cast<double *>(a.sc + i) + r; y = reinterpret_cast<double *>(a.sc + j) + r;
         } else if ((r -= eS) < eA) {
             x = a.A + i * a.sA + r; y = a.A + j * a.sA + r;
+        } else if ((r -= eA) >= eQ) {
+            r -= eQ;
+            x = a.vb + (long long)i * a.nvb + r; y = a.vb + (long long)j * a.nvb + r;
         } else {
-            r -= eA;
             const long long arr = r / a.neq, k = r % a.neq;
             double *base = a.veq + arr * (long long)a.Btot * a.neq;
             x = base + (long long)i * a.neq + k; y = base + (long long)j * a.neq + k;
@@ -267,12 +507,21 @@ __global__ void k_transpose_A(const double *A, long long lda, long long sA, doub
         At[b * sAt + i + k * ldas] = A[b * sA + k + i * lda];
     }
 }
-// NT scaling at iteration 0 (misc.py:284-287) and lambda^2 (:2244)
+// NT scaling at iteration 0 (misc.py:284-287, 'q': :311-354) and lambda^2 (:2244)
+template <class Gp>
 __global__ void k_scaling(Ptrs p, int first) {
     PB_SETUP
-    (void)sh; (void)on;
+    (void)on;
     if (S.done) return;
-    for (int i = tid; i < p.m; i += nt) {
+    if (p.c.nq > 0) {
+        const Gp g;
+        Q_LOOP(g) {
+            Q_CONE(k)
+            if (first) q_compute_scaling(g, p.s + oq, p.z + oq, vq_, betaq_, p.lmbda + oq, mq, sh);
+            q_ssqr(g, p.lmbdasq + oq, p.lmbda + oq, mq, sh);
+        }
+    }
+    for (int i = tid; i < p.c.ml; i += nt) {
         if (first) {
             const double sv = p.s[om + i], zv = p.z[om + i];
             const double d = sqrt(sv / zv);
@@ -285,33 +534,177 @@ __global__ void k_scaling(Ptrs p, int first) {
         const double l = p.lmbda[om + i];
         p.lmbdasq[om + i] = l * l;
     }
-    if (tid == 0) { S.mu = S.gap / p.m; S.sigma = 0.0; S.eta = 0.0; }       // :2357-2358
+    if (tid == 0) { S.mu = S.gap / (p.c.ml + p.c.nq); S.sigma = 0.0; S.eta = 0.0; }       // :2357-2358
 }
-// right-hand side of the i-th Newton system and the f4_no_ir preamble (:2376-2309)
-__global__ void k_dir_prep(Ptrs p, int i) {
+// f4_no_ir's preamble for one cone (:2303-2309): s := lambda o\ s, z := z - W's, bzp := W^{-T} z for the solve
+template <class Gp>
+__device__ void q_f4_pre(const Gp &g, const Ptrs &p, long long oq, const double *v, double beta, int mq,
+                         double *zv, double *sv, double *sh) {
+    q_sinv(g, sv + oq, p.lmbda + oq, mq, sh);
+    for (int j = g.rank(); j < mq; j += g.size()) p.bzp[oq + j] = sv[oq + j];
+    g.sync();
+    q_scale(g, p.bzp + oq, v, beta, mq, false, sh);                  // W' = W for 'q'
+    for (int j = g.rank(); j < mq; j += g.size()) {
+        const double t = zv[oq + j] - p.bzp[oq + j];
+        zv[oq + j] = t;
+        p.bzp[oq + j] = t;
+    }
+    g.sync();
+    q_scale(g, p.bzp + oq, v, beta, mq, true, sh);
+}
+// right-hand side of the i-th Newton system and the f4_no_ir preamble (:2376-2309); save: keep the right-hand side
+// for iterative refinement (f4, :2330-2336)
+template <class Gp>
+__global__ void k_dir_prep(Ptrs p, int i, int save) {
     PB_SETUP
-    (void)sh;
     const double sm = S.sigma * S.mu, c = -1.0 + S.eta;
-    for (int k = tid; k < p.n; k += nt) p.dx[on + k] = c * p.rx[on + k];
+    for (int k = tid; k < p.n; k += nt) {
+        const double v = c * p.rx[on + k];
+        p.dx[on + k] = v;
+        if (save) p.wx[on + k] = v;
+    }
     const long long op = (long long)b * p.neq;
-    for (int k = tid; k < p.neq; k += nt) p.dy[op + k] = c * p.ry[op + k];
-    for (int k = tid; k < p.m; k += nt) {
+    for (int k = tid; k < p.neq; k += nt) {
+        const double v = c * p.ry[op + k];
+        p.dy[op + k] = v;
+        if (save) p.wy[op + k] = v;
+    }
+    for (int k = tid; k < p.c.ml; k += nt) {
         double ds = -p.lmbdasq[om + k] + sm;
         if (i == 1) ds -= p.ws3[om + k];                 // Mehrotra correction
+        if (save) { p.ws[om + k] = ds; p.wz[om + k] = c * p.rz[om + k]; }
         ds = ds / p.lmbda[om + k];                       // sinv
         p.ds[om + k] = ds;
         const double dz = c * p.rz[om + k] - p.d[om + k] * ds;   // z := z - W' s
         p.dz[om + k] = dz;
         p.bzp[om + k] = p.di[om + k] * dz;               // W^{-T} bz for the solve
     }
+    if (p.c.nq > 0) {
+        const Gp g;
+        Q_LOOP(g) {
+            Q_CONE(k)
+            for (int j = g.rank(); j < mq; j += g.size()) {
+                // ds = -lambda o lambda (- ws3) + sigma mu e  (:2376-2385)
+                double ds = -p.lmbdasq[oq + j] + sm * p.c.e[p.c.off[k] + j];
+                if (i == 1) ds -= p.ws3[oq + j];
+                const double bz = c * p.rz[oq + j];
+                p.ds[oq + j] = ds;
+                p.dz[oq + j] = bz;
+                if (save) { p.ws[oq + j] = ds; p.wz[oq + j] = bz; }
+            }
+            g.sync();
+            q_f4_pre(g, p, oq, vq_, *betaq_, mq, p.dz, p.ds, sh);
+        }
+    }
 }
-// after the solve: dz = bzp (= W uz); ds := ds - dz; step length, sigma (:2316, :2423-2456)
-__global__ void k_dir_post(Ptrs p, int i) {
+// refinement: the preamble of f4_no_ir on the correction's right-hand side (z2, s2)
+template <class Gp>
+__global__ void k_f4_pre(Ptrs p) {
     PB_SETUP
-    double dsdz = 0, mins = INFINITY, minz = INFINITY;
+    (void)on; (void)S;
+    for (int k = tid; k < p.c.ml; k += nt) {
+        const double s = p.s2[om + k] / p.lmbda[om + k];
+        p.s2[om + k] = s;
+        const double z = p.z2[om + k] - p.d[om + k] * s;
+        p.z2[om + k] = z;
+        p.bzp[om + k] = p.di[om + k] * z;
+    }
+    if (p.c.nq > 0) {
+        const Gp g;
+        Q_LOOP(g) {
+            Q_CONE(k)
+            q_f4_pre(g, p, oq, vq_, *betaq_, mq, p.z2, p.s2, sh);
+        }
+    }
+}
+// refinement: f4_no_ir's end (:2316) for the first solution: dz := uz (bzp), ds := ds - dz
+__global__ void k_f4_post(Ptrs p) {
+    PB_SETUP
+    (void)sh; (void)S; (void)on;
     for (int k = tid; k < p.m; k += nt) {
         const double dz = p.bzp[om + k];
-        const double ds = p.ds[om + k] - dz;
+        p.dz[om + k] = dz;
+        p.ds[om + k] -= dz;
+    }
+}
+// refinement, res() (:1930-1960):  x2 = wx, y2 = wy (the GEMVs subtract P dx + A'dy + G'W^{-1}dz and A dx),
+// t3 = W^{-1} dz,  z2 = wz - W'ds (the GEMV subtracts G dx),  s2 = ws - lambda o (dz + ds)
+template <class Gp>
+__global__ void k_res_prep(Ptrs p) {
+    PB_SETUP
+    (void)S;
+    for (int k = tid; k < p.n; k += nt) p.x2[on + k] = p.wx[on + k];
+    const long long op = (long long)b * p.neq;
+    for (int k = tid; k < p.neq; k += nt) p.y2[op + k] = p.wy[op + k];
+    for (int k = tid; k < p.c.ml; k += nt) {
+        const double uz = p.dz[om + k], us = p.ds[om + k];
+        p.t3[om + k] = p.di[om + k] * uz;
+        p.z2[om + k] = p.wz[om + k] - p.d[om + k] * us;
+        p.s2[om + k] = p.ws[om + k] - p.lmbda[om + k] * (us + uz);
+    }
+    if (p.c.nq > 0) {
+        const Gp g;
+        Q_LOOP(g) {
+            Q_CONE(k)
+            for (int j = g.rank(); j < mq; j += g.size()) {
+                const double uz = p.dz[oq + j], us = p.ds[oq + j];
+                p.t3[oq + j] = uz; p.z2[oq + j] = us; p.s2[oq + j] = us + uz;
+            }
+            g.sync();
+            q_scale(g, p.t3 + oq, vq_, *betaq_, mq, true, sh);
+            q_scale(g, p.z2 + oq, vq_, *betaq_, mq, false, sh);
+            q_sprod(g, p.s2 + oq, p.lmbda + oq, mq, sh);          // sprod(.., diag='D') is the same for 'q'
+            for (int j = g.rank(); j < mq; j += g.size()) {
+                p.z2[oq + j] = p.wz[oq + j] - p.z2[oq + j];
+                p.s2[oq + j] = p.ws[oq + j] - p.s2[oq + j];
+            }
+            g.sync();
+        }
+    }
+}
+// refinement: dx += x2, dy += y2, dz += uz2, ds += s2 - uz2  (:2343-2347 after f4_no_ir's :2316)
+__global__ void k_ref_add(Ptrs p) {
+    PB_SETUP
+    (void)sh; (void)S;
+    for (int k = tid; k < p.n; k += nt) p.dx[on + k] += p.x2[on + k];
+    const long long op = (long long)b * p.neq;
+    for (int k = tid; k < p.neq; k += nt) p.dy[op + k] += p.y2[op + k];
+    for (int k = tid; k < p.m; k += nt) {
+        const double uz = p.bzp[om + k];
+        p.dz[om + k] += uz;
+        p.ds[om + k] += p.s2[om + k] - uz;
+    }
+}
+// after the solve: dz = bzp (= W uz); ds := ds - dz (done already when refined); step length, sigma
+// (:2316, :2423-2456)
+template <class Gp>
+__global__ void k_dir_post(Ptrs p, int i, int refined) {
+    PB_SETUP
+    double dsdz = 0, mins = INFINITY, minz = INFINITY;
+    double tq = -INFINITY;                               // max_step over the cones
+    if (p.c.nq > 0) {
+        const Gp g;
+        Q_LOOP(g) {
+            Q_CONE(k) (void)vq_; (void)betaq_;
+            for (int j = g.rank(); j < mq; j += g.size()) {
+                const double dz = refined ? p.dz[oq + j] : p.bzp[oq + j];
+                const double ds = refined ? p.ds[oq + j] : p.ds[oq + j] - dz;
+                p.dz[oq + j] = dz; p.ds[oq + j] = ds;
+                dsdz += ds * dz;
+                if (i == 0) p.ws3[oq + j] = ds;
+            }
+            g.sync();
+            if (i == 0) q_sprod(g, p.ws3 + oq, p.dz + oq, mq, sh);   // ws3 = ds o dz (:2426-2428)
+            q_scale2(g, p.lmbda + oq, p.ds + oq, mq, false, sh);
+            q_scale2(g, p.lmbda + oq, p.dz + oq, mq, false, sh);
+            const double t1 = q_max_step(g, p.ds + oq, mq, sh);
+            const double t2 = q_max_step(g, p.dz + oq, mq, sh);
+            tq = fmax(tq, fmax(t1, t2));
+        }
+    }
+    for (int k = tid; k < p.c.ml; k += nt) {
+        const double dz = refined ? p.dz[om + k] : p.bzp[om + k];
+        const double ds = refined ? p.ds[om + k] : p.ds[om + k] - dz;
         dsdz += ds * dz;
         if (i == 0) p.ws3[om + k] = ds * dz;
         const double l = p.lmbda[om + k];
@@ -322,8 +715,10 @@ __global__ void k_dir_post(Ptrs p, int i) {
     dsdz = block_sum(dsdz, sh);
     mins = block_min(mins, sh);
     minz = block_min(minz, sh);
+    if (p.c.nq > 0) tq = block_max(tq, sh);
     if (tid == 0) {
-        const double t = fmax(0.0, fmax(-mins, -minz));
+        double t = fmax(0.0, fmax(-mins, -minz));
+        if (p.c.nq > 0) t = fmax(t, tq);
         double step;
         if (t == 0.0) step = 1.0;
         else step = (i == 0) ? fmin(1.0, 1.0 / t) : fmin(1.0, 0.99 / t);
@@ -335,7 +730,8 @@ __global__ void k_dir_post(Ptrs p, int i) {
         }
     }
 }
-// x += step dx; new scaled iterates, scaling update, unscaled s, z, gap (:2459-2547, misc.py:450-464)
+// x += step dx; new scaled iterates, scaling update, unscaled s, z, gap (:2459-2547, misc.py:450-464, 'q': :504-573)
+template <class Gp>
 __global__ void k_update(Ptrs p, const int *info, int iter) {
     PB_SETUP
     if (S.done) return;
@@ -348,7 +744,7 @@ __global__ void k_update(Ptrs p, const int *info, int iter) {
     const long long op = (long long)b * p.neq;
     for (int k = tid; k < p.neq; k += nt) p.y[op + k] += step * p.dy[op + k];
     double gap = 0;
-    for (int k = tid; k < p.m; k += nt) {
+    for (int k = tid; k < p.c.ml; k += nt) {
         const double l = p.lmbda[om + k];
         const double ds = (1.0 + step * p.ds[om + k]) * l;      // scale2 inverse
         const double dz = (1.0 + step * p.dz[om + k]) * l;
@@ -362,8 +758,61 @@ __global__ void k_update(Ptrs p, const int *info, int iter) {
         p.z[om + k] = di * ln;                                  // W^{-1} lambda
         gap += ln * ln;
     }
+    if (p.c.nq > 0) {
+        const Gp g;
+        Q_LOOP(g) {
+            Q_CONE(k)
+            const double *e = p.c.e + p.c.off[k];
+            for (int j = g.rank(); j < mq; j += g.size()) {       // ds := e + step ds, dz := e + step dz
+                p.ds[oq + j] = step * p.ds[oq + j] + e[j];
+                p.dz[oq + j] = step * p.dz[oq + j] + e[j];
+            }
+            g.sync();
+            q_scale2(g, p.lmbda + oq, p.ds + oq, mq, true, sh);
+            q_scale2(g, p.lmbda + oq, p.dz + oq, mq, true, sh);
+            q_update_scaling(g, p.ds + oq, p.dz + oq, vq_, betaq_, p.lmbda + oq, mq, sh);
+            for (int j = g.rank(); j < mq; j += g.size()) {
+                const double l = p.lmbda[oq + j];
+                p.s[oq + j] = l; p.z[oq + j] = l;
+                gap += l * l;
+            }
+            g.sync();
+            q_scale(g, p.s + oq, vq_, *betaq_, mq, false, sh);      // s = W' lambda
+            q_scale(g, p.z + oq, vq_, *betaq_, mq, true, sh);       // z = W^{-1} lambda
+        }
+    }
     gap = block_sum(gap, sh);
     if (tid == 0) S.gap = gap;
+}
+
+// Gs_q := W^{-T} G_q for every problem (blockIdx.y), column and cone: the 'q' rows of the scaled G whose Gram matrix
+// enters S = P + G' W^{-1} W^{-T} G (kkt_chol2 / kkt_chol, misc.py:1407-1418).  Same arithmetic as scale_q_kernel
+// (cone.cu) with inverse; W is symmetric.  One thread (cones of <= 8 rows) or one warp per (column, cone); cones
+// vary fastest, so the threads of a warp read neighbouring rows of a column.
+template <bool PerThread>
+__global__ void k_scale_gq(Ptrs p, const double *G, long long ldg, long long sG, double *Gs, long long ldgs,
+                           long long sGs) {
+    constexpr int per = PerThread ? 1 : 32;
+    const long long b = blockIdx.y;
+    const long long item = ((long long)blockIdx.x * blockDim.x + threadIdx.x) / per;
+    const int lane = PerThread ? 0 : (threadIdx.x & 31);
+    if (item >= (long long)p.n * p.c.nq) return;
+    const int k = (int)(item % p.c.nq);
+    const long long j = item / p.c.nq;
+    const int mq = p.c.dim[k];
+    const double *x = G + b * sG + j * ldg + p.c.ml + p.c.off[k];
+    double *y = Gs + b * sGs + j * ldgs + p.c.off[k];
+    const double *vb = p.c.vb + b * (p.c.sumq + p.c.nq);
+    const double *v = vb + p.c.off[k];
+    double w = 0;
+    for (int i = lane; i < mq; i += per) w += v[i] * (i == 0 ? -x[i] : x[i]);
+    if (!PerThread) w = warp_sum(w);
+    const double tw = 2.0 * w, bi = 1.0 / vb[p.c.sumq + k];
+    for (int i = lane; i < mq; i += per) {
+        double yi = x[i] + v[i] * tw;
+        if (i == 0) yi = -yi;
+        y[i] = yi * bi;
+    }
 }
 
 }  // namespace
@@ -388,6 +837,19 @@ struct cvxb_batch {
     bool time_phases = false;
     double phase_ms[3] = {0, 0, 0};  // S: SYRK + Cholesky; TRSM (Asct); Kp: SYRK + Cholesky
     cudaEvent_t ph[4] = {nullptr, nullptr, nullptr, nullptr};
+    double qphase_ms[2] = {0, 0};    // within S: the Gs_q scaling; the GEMM K += Gs_q' Gs_q
+    cudaEvent_t qph[3] = {nullptr, nullptr, nullptr};
+    // 'q' cones (dims = {'l': ml, 'q': qdim}; m = ml + sumq).  Nothing below is allocated without cones.
+    int ml = 0, nq = 0, sumq = 0;
+    int qmode = 0;                   // threads per cone in the cone kernels: 0 one, 1 a warp, 2 the CTA
+    std::vector<int> qdim;
+    int *d_qtab = nullptr;           // dim[nq], off[nq]
+    double *qe = nullptr;            // sumq: the cones' identity e
+    double *vb = nullptr;            // per problem: v (sumq), beta (nq)
+    double *Gs = nullptr;            // per problem: W^{-T} G_q, sumq x n (ld ldgs)
+    long long ldgs = 0, sGs = 0;
+    // iterative refinement workspace, allocated by the first solve that refines
+    double *refw = nullptr;
     double *K = nullptr, *inv = nullptr, *panel = nullptr, *gemv_ws = nullptr;
     double *vecs = nullptr;          // all n- and m-vectors
     Ptrs p;
@@ -427,15 +889,30 @@ void phase_add(cvxb_batch *b, int k) {
     cudaGetLastError();
 }
 
-// K := P + G' diag(di)^2 G (+ A' diag(wsing) A where flagged) and its Cholesky factor; d_info per problem
+void qphase(cvxb_batch *b, int k) {
+    if (b->time_phases) cudaEventRecord(b->qph[k], b->st);
+}
+
+// launch a cone kernel with the batch's group size per cone (GThread / GWarp / GBlock)
+#define QLAUNCH(kern, grid, T, st, ...) do {                                         \
+        switch (b->qmode) {                                                          \
+        case 1: kern<GWarp><<<(grid), (T), 0, (st)>>>(__VA_ARGS__); break;           \
+        case 2: kern<GBlock><<<(grid), (T), 0, (st)>>>(__VA_ARGS__); break;          \
+        default: kern<GThread><<<(grid), (T), 0, (st)>>>(__VA_ARGS__); break;        \
+        }                                                                            \
+        count_launch();                                                              \
+    } while (0)
+
+// K := P + G_l' diag(di)^2 G_l + Gs_q' Gs_q (+ A' diag(wsing) A where flagged) and its Cholesky factor;
+// d_info per problem
 int factor_S(cvxb_batch *b, bool i8) {
     cudaStream_t st = b->st;
     if (i8) {
-        CVXB_TRY(ozaki_syrk(b->n, b->m, b->G, b->ldg, b->p.di, b->P, b->ldp, 1.0, b->K, b->ldk, 9, 0,
+        CVXB_TRY(ozaki_syrk(b->n, b->ml, b->G, b->ldg, b->p.di, b->P, b->ldp, 1.0, b->K, b->ldk, 9, 0,
                             b->oz_work, nullptr, st));
-    } else {
+    } else if (b->ml > 0 || b->nq == 0) {
         GemmDesc g;
-        g.M = b->n; g.N = b->n; g.K = b->m;
+        g.M = b->n; g.N = b->n; g.K = b->ml;
         g.X = b->G; g.ldx = (int)b->ldg; g.x_kmajor = true; g.sX = b->sG;
         g.Y = b->G; g.ldy = (int)b->ldg; g.y_kmajor = true; g.sY = b->sG;
         g.w = b->p.di2; g.sW = b->m;
@@ -444,6 +921,37 @@ int factor_S(cvxb_batch *b, bool i8) {
         g.lower_only = true; g.batch = b->Bact;
         if (b->B == 1) g.splitk_ws = b->cw.splitk_ws;
         CVXB_TRY(dmma_gemm(g, st));
+    }
+    if (b->nq > 0) {
+        // Gs_q = W^{-T} G_q, then K += Gs_q' Gs_q (K := P + Gs_q' Gs_q without 'l' rows), as cvxb_kkt_factor does
+        // for its non-'l' rows
+        qphase(b, 0);
+        const bool per_thread = b->qmode == 0;
+        const long long items = (long long)b->n * b->nq, per_block = per_thread ? 256 : 8;
+        const dim3 grid((unsigned)((items + per_block - 1) / per_block), (unsigned)b->Bact);
+        if (per_thread) k_scale_gq<true><<<grid, 256, 0, st>>>(b->p, b->G, b->ldg, b->sG, b->Gs, b->ldgs, b->sGs);
+        else k_scale_gq<false><<<grid, 256, 0, st>>>(b->p, b->G, b->ldg, b->sG, b->Gs, b->ldgs, b->sGs);
+        count_launch();
+        CVXB_LAUNCH_CHECK();
+        qphase(b, 1);
+        GemmDesc g;
+        g.M = b->n; g.N = b->n; g.K = b->sumq;
+        g.X = b->Gs; g.ldx = (int)b->ldgs; g.x_kmajor = true; g.sX = b->sGs;
+        g.Y = b->Gs; g.ldy = (int)b->ldgs; g.y_kmajor = true; g.sY = b->sGs;
+        if (b->ml > 0 || i8) { g.D = b->K; g.ldd = (int)b->ldk; g.sD = b->sK; }
+        else { g.D = b->P; g.ldd = (int)b->ldp; g.sD = b->sP; }
+        g.beta = 1.0;
+        g.C = b->K; g.ldc = (int)b->ldk; g.sC = b->sK;
+        g.lower_only = true; g.batch = b->Bact;
+        CVXB_TRY(dmma_gemm(g, st));
+        qphase(b, 2);
+        if (b->time_phases) {
+            float t = 0;
+            cudaEventSynchronize(b->qph[2]);
+            if (cudaEventElapsedTime(&t, b->qph[0], b->qph[1]) == cudaSuccess) b->qphase_ms[0] += t;
+            if (cudaEventElapsedTime(&t, b->qph[1], b->qph[2]) == cudaSuccess) b->qphase_ms[1] += t;
+            cudaGetLastError();
+        }
     }
     if (b->nsing > 0) {
         // K += A' diag(wsing) A: adds A'A to the flagged problems' S and exactly zero to the others (misc.py:1452-1454)
@@ -500,11 +1008,11 @@ int factor_eq(cvxb_batch *b) {
 
 // first: the factorisation at the starting point (W = I), where kkt_chol2 decides which problems are singular
 int batch_factor(cvxb_batch *b, bool first = false) {
-    bool i8 = b->B == 1 && b->m > 0 && (b->i8_mode == 2 || (b->i8_mode == 1 && b->n >= 4096 && b->m >= 8192));
+    bool i8 = b->B == 1 && b->ml > 0 && (b->i8_mode == 2 || (b->i8_mode == 1 && b->n >= 4096 && b->ml >= 8192));
     if (i8) {
-        // K = P + G' diag(di)^2 G from nine int8 slices per entry (fp64-accurate, ~1.8x the DMMA SYRK);
+        // K = P + G_l' diag(di)^2 G_l from nine int8 slices per entry (fp64-accurate, ~1.8x the DMMA SYRK);
         // same size rule and same fallback (workspace does not fit -> DMMA kernel) as cvxb_kkt_factor
-        const size_t need = ozaki_workspace_bytes(b->n, b->m, 9);
+        const size_t need = ozaki_workspace_bytes(b->n, b->ml, 9);
         if (need > b->oz_bytes) {
             if (b->oz_work) cudaFree(b->oz_work);
             b->oz_work = nullptr; b->oz_bytes = 0;
@@ -536,32 +1044,42 @@ int batch_factor(cvxb_batch *b, bool first = false) {
     return 0;
 }
 
-// (dx, dy, bzp) := solution of the reduced KKT system; on entry dx = bx, dy = by, bzp = W^{-T} bz
-int batch_solve(cvxb_batch *b) {
+// (x, y, bzp) := solution of the reduced KKT system; on entry x = bx, y = by, bzp = W^{-T} bz
+int batch_solve(cvxb_batch *b, double *x, double *y) {
     cudaStream_t st = b->st;
-    const int n = b->n, m = b->m, B = b->Bact, pe = b->neq;
+    const int n = b->n, m = b->m, B = b->Bact, pe = b->neq, ml = b->ml;
+    double *bzq = b->p.bzp + ml;                 // the 'q' rows of bzp
     GemvBatch gt; gt.batch = B; gt.sA = b->sG; gt.sw = m; gt.sx = m; gt.sy = n;
-    // x := x + G' (di .* bzp)
-    CVXB_TRY(gemv_t(m, n, b->G, b->ldg, b->p.di, b->p.bzp, 1.0, 1.0, b->p.dx, st, gt));
+    // x := x + G_l' (di .* bzp_l) + Gs_q' bzp_q
+    if (ml > 0 || b->nq == 0) CVXB_TRY(gemv_t(ml, n, b->G, b->ldg, b->p.di, b->p.bzp, 1.0, 1.0, x, st, gt));
+    if (b->nq > 0) {
+        GemvBatch gq; gq.batch = B; gq.sA = b->sGs; gq.sx = m; gq.sy = n;
+        CVXB_TRY(gemv_t(b->sumq, n, b->Gs, b->ldgs, nullptr, bzq, 1.0, 1.0, x, st, gq));
+    }
     if (pe == 0) {
-        CVXB_TRY(potrs_lower(n, b->K, (int)b->ldk, b->inv, b->p.dx, b->cw, st, B, b->sK, b->sInv, n));
+        CVXB_TRY(potrs_lower(n, b->K, (int)b->ldk, b->inv, x, b->cw, st, B, b->sK, b->sInv, n));
     } else {
         // kkt_chol2's solve (misc.py:1526-1558)
         if (b->nsing > 0) {       // x += A' by where S + A'A is factored
             GemvBatch ga; ga.batch = B; ga.sA = b->sA; ga.sw = pe; ga.sx = pe; ga.sy = n;
-            CVXB_TRY(gemv_t(pe, n, b->A, b->lda, b->p.wsing, b->p.dy, 1.0, 1.0, b->p.dx, st, ga));
+            CVXB_TRY(gemv_t(pe, n, b->A, b->lda, b->p.wsing, y, 1.0, 1.0, x, st, ga));
         }
-        CVXB_TRY(trsv_lower(n, b->K, (int)b->ldk, b->inv, b->p.dx, false, b->cw, st, B, b->sK, b->sInv, n));
+        CVXB_TRY(trsv_lower(n, b->K, (int)b->ldk, b->inv, x, false, b->cw, st, B, b->sK, b->sInv, n));
         GemvBatch gyt; gyt.batch = B; gyt.sA = b->sAs; gyt.sx = n; gyt.sy = pe;       // y := Asct' x - y
-        CVXB_TRY(gemv_t(n, pe, b->Asct, b->ldk, nullptr, b->p.dx, 1.0, -1.0, b->p.dy, st, gyt));
-        CVXB_TRY(potrs_lower(pe, b->Kp, (int)b->ldkp, b->invp, b->p.dy, b->cw, st, B, b->sKp, b->sInvp, pe));
+        CVXB_TRY(gemv_t(n, pe, b->Asct, b->ldk, nullptr, x, 1.0, -1.0, y, st, gyt));
+        CVXB_TRY(potrs_lower(pe, b->Kp, (int)b->ldkp, b->invp, y, b->cw, st, B, b->sKp, b->sInvp, pe));
         GemvBatch gyn; gyn.batch = B; gyn.sA = b->sAs; gyn.sx = pe; gyn.sy = n;       // x -= Asct y
-        CVXB_TRY(gemv_n(n, pe, b->Asct, b->ldk, nullptr, b->p.dy, -1.0, 1.0, b->p.dx, b->gemv_ws, st, gyn));
-        CVXB_TRY(trsv_lower(n, b->K, (int)b->ldk, b->inv, b->p.dx, true, b->cw, st, B, b->sK, b->sInv, n));
+        CVXB_TRY(gemv_n(n, pe, b->Asct, b->ldk, nullptr, y, -1.0, 1.0, x, b->gemv_ws, st, gyn));
+        CVXB_TRY(trsv_lower(n, b->K, (int)b->ldk, b->inv, x, true, b->cw, st, B, b->sK, b->sInv, n));
     }
-    // bzp := di .* (G x) - bzp
+    // bzp := [di .* (G_l x); Gs_q x] - bzp
     GemvBatch gn; gn.batch = B; gn.sA = b->sG; gn.sw = m; gn.sx = n; gn.sy = m;
-    CVXB_TRY(gemv_n(m, n, b->G, b->ldg, b->p.di, b->p.dx, 1.0, -1.0, b->p.bzp, b->gemv_ws, st, gn));
+    if (ml > 0 || b->nq == 0)
+        CVXB_TRY(gemv_n(ml, n, b->G, b->ldg, b->p.di, x, 1.0, -1.0, b->p.bzp, b->gemv_ws, st, gn));
+    if (b->nq > 0) {
+        GemvBatch gq; gq.batch = B; gq.sA = b->sGs; gq.sx = n; gq.sy = m;
+        CVXB_TRY(gemv_n(b->sumq, n, b->Gs, b->ldgs, nullptr, x, 1.0, -1.0, bzq, b->gemv_ws, st, gq));
+    }
     return 0;
 }
 
@@ -574,7 +1092,21 @@ int cvxb_batch_create(cvxb_batch **out, int nprob, int n, int m, int device) {
 }
 
 int cvxb_batch_create_eq(cvxb_batch **out, int nprob, int n, int m, int p, int device) {
-    if (!out || nprob <= 0 || n <= 0 || m < 0) { set_error("batch_create: bad sizes"); return CVXB_E_ARG; }
+    return cvxb_batch_create_cones(out, nprob, n, m, 0, nullptr, p, device);
+}
+
+int cvxb_batch_create_cones(cvxb_batch **out, int nprob, int n, int ml, int nq, const int *qdims, int p, int device) {
+    if (!out || nprob <= 0 || n <= 0 || ml < 0) { set_error("batch_create: bad sizes"); return CVXB_E_ARG; }
+    if (nq < 0 || (nq > 0 && !qdims)) { set_error("batch_create: bad 'q' cone list"); return CVXB_E_ARG; }
+    long long msum = ml;
+    int qmax = 0;
+    for (int k = 0; k < nq; ++k) {
+        if (qdims[k] < 1) { set_error("batch_create: 'q' cone %d has size %d (must be >= 1)", k, qdims[k]); return CVXB_E_ARG; }
+        msum += qdims[k];
+        qmax = std::max(qmax, qdims[k]);
+    }
+    if (msum > (1 << 30)) { set_error("batch_create: bad sizes"); return CVXB_E_ARG; }
+    const int m = (int)msum;
     if (p < 0 || p > n) { set_error("batch_create: need 0 <= p <= n (p = %d, n = %d)", p, n); return CVXB_E_ARG; }
     if (p > 0 && m == 0) { set_error("batch_create: equality constraints need m > 0"); return CVXB_E_ARG; }
     *out = nullptr;
@@ -588,6 +1120,11 @@ int cvxb_batch_create_eq(cvxb_batch **out, int nprob, int n, int m, int p, int d
     CVXB_CUDA(cudaSetDevice(device));
     cvxb_batch *b = new cvxb_batch();
     b->device = device; b->B = nprob; b->n = n; b->m = m; b->neq = p;
+    b->ml = ml; b->nq = nq; b->sumq = m - ml;
+    b->qdim.assign(qdims, qdims + nq);
+    // one thread per cone for cones of <= 8 rows, a warp per cone when there are enough of them to fill the CTA,
+    // else the whole CTA per cone (a few large cones)
+    b->qmode = qmax <= 8 ? 0 : (nq >= 256 / 32 ? 1 : 2);
     if (const char *e = getenv("CVXB_OZAKI")) b->i8_mode = (e[0] == '0') ? 0 : (e[0] == '2') ? 2 : 1;
     if (const char *e = getenv("CVXB_OZAKI_IPM")) b->i8_mode = (e[0] == '1') ? 1 : (e[0] == '2') ? 2 : 0;
     b->ldg = ((m + 1) & ~1) > 2 ? ((m + 1) & ~1) : 2;
@@ -628,6 +1165,24 @@ int cvxb_batch_create_eq(cvxb_batch **out, int nprob, int n, int m, int p, int d
     b->p.di = take(me); b->p.di2 = take(me); b->p.ws3 = take(me); b->p.bzp = take(me);
     b->p.q = b->q; b->p.h = b->h; b->p.n = n; b->p.m = m;
     b->p.neq = p; b->p.beq = nullptr; b->p.y = b->p.ry = b->p.dy = b->p.wsing = nullptr;
+    b->p.wx = b->p.wy = b->p.wz = b->p.ws = b->p.x2 = b->p.y2 = b->p.z2 = b->p.s2 = b->p.t3 = nullptr;
+    b->p.c.ml = ml; b->p.c.nq = nq; b->p.c.sumq = b->sumq;
+    b->p.c.dim = b->p.c.off = nullptr; b->p.c.e = nullptr; b->p.c.vb = nullptr;
+    if (nq > 0) {
+        std::vector<int> tab(2 * (size_t)nq);
+        std::vector<double> e((size_t)b->sumq, 0.0);
+        for (int k = 0, o = 0; k < nq; o += qdims[k], ++k) { tab[k] = qdims[k]; tab[nq + k] = o; e[o] = 1.0; }
+        BCUDA(cudaMalloc(&b->d_qtab, tab.size() * sizeof(int)));
+        BCUDA(cudaMemcpy(b->d_qtab, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice));
+        BCUDA(cudaMalloc(&b->qe, e.size() * sizeof(double)));
+        BCUDA(cudaMemcpy(b->qe, e.data(), e.size() * sizeof(double), cudaMemcpyHostToDevice));
+        BCUDA(cudaMalloc(&b->vb, B * (size_t)(b->sumq + nq) * sizeof(double)));
+        BCUDA(cudaMemset(b->vb, 0, B * (size_t)(b->sumq + nq) * sizeof(double)));
+        b->ldgs = std::max<long long>(2, (b->sumq + 1) & ~1);
+        b->sGs = b->ldgs * n;
+        BCUDA(cudaMalloc(&b->Gs, B * b->sGs * sizeof(double)));
+        b->p.c.dim = b->d_qtab; b->p.c.off = b->d_qtab + nq; b->p.c.e = b->qe; b->p.c.vb = b->vb;
+    }
     if (p > 0) {
         b->lda = b->ldkp = (p + 1) & ~1;
         b->sA = b->lda * n; b->sAs = b->ldk * p; b->sKp = b->ldkp * p;
@@ -644,8 +1199,10 @@ int cvxb_batch_create_eq(cvxb_batch **out, int nprob, int n, int m, int p, int d
         b->p.beq = w; b->p.y = w + B * p; b->p.ry = w + 2 * B * p; b->p.dy = w + 3 * B * p; b->p.wsing = w + 4 * B * p;
     }
     if (const char *e = getenv("CVXB_BATCH_PHASE_MS")) b->time_phases = e[0] == '1';
-    if (b->time_phases)
+    if (b->time_phases) {
         for (cudaEvent_t &e : b->ph) BCUDA(cudaEventCreate(&e));
+        for (cudaEvent_t &e : b->qph) BCUDA(cudaEventCreate(&e));
+    }
     BCUDA(cudaMalloc(&b->sc, B * sizeof(Scal)));
     BCUDA(cudaMemset(b->sc, 0, B * sizeof(Scal)));
     b->p.sc = b->sc;
@@ -666,8 +1223,11 @@ void cvxb_batch_destroy(cvxb_batch *b) {
     if (!b) return;
     cudaSetDevice(b->device);
     if (b->st) cudaStreamSynchronize(b->st);
-    double *bufs[] = {b->P, b->G, b->K, b->inv, b->panel, b->gemv_ws, b->vecs, b->A, b->Asct, b->Kp, b->invp, b->veq};
+    double *bufs[] = {b->P, b->G, b->K, b->inv, b->panel, b->gemv_ws, b->vecs, b->A, b->Asct, b->Kp, b->invp, b->veq,
+                      b->qe, b->vb, b->Gs, b->refw};
     for (double *x : bufs) if (x) cudaFree(x);
+    if (b->d_qtab) cudaFree(b->d_qtab);
+    for (cudaEvent_t e : b->qph) if (e) cudaEventDestroy(e);
     if (b->d_infop) cudaFree(b->d_infop);
     if (b->d_nsing) cudaFree(b->d_nsing);
     for (cudaEvent_t e : b->ph) if (e) cudaEventDestroy(e);
@@ -720,6 +1280,7 @@ static int swap_slots(cvxb_batch *b, const std::vector<int> &pairs) {
     a.P = b->P; a.G = b->G; a.vecs = b->vecs; a.sc = b->sc; a.sP = b->sP; a.sG = b->sG;
     a.n = b->n; a.me = b->m > 0 ? b->m : 1; a.Btot = b->B;
     a.A = b->A; a.veq = b->veq; a.sA = b->sA; a.neq = b->neq;
+    a.vb = b->vb; a.nvb = b->nq > 0 ? b->sumq + b->nq : 0;
     k_swap_slots<<<dim3(96, np), 256, 0, b->st>>>(a, b->d_pairs);
     count_launch();
     // `pairs` is pageable host memory: the copy above is staged before cudaMemcpyAsync returns
@@ -762,12 +1323,36 @@ int cvxb_batch_load_eq(cvxb_batch *b, const double *A, const double *bvec, int s
 }
 
 int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, double feastol) {
+    return cvxb_batch_solve_ref(b, maxiters, abstol, reltol, feastol, -1);
+}
+
+int cvxb_batch_solve_ref(cvxb_batch *b, int maxiters, double abstol, double reltol, double feastol, int refinement) {
     if (!b || !b->loaded) { set_error("batch_solve: load the problems first"); return CVXB_E_ARG; }
+    // coneqp's default: one step of iterative refinement when there are 'q' cones, none otherwise (:1862-1865)
+    const int refine = refinement >= 0 ? refinement : (b->nq > 0 ? 1 : 0);
     if (b->neq > 0 && !b->eq_loaded) { set_error("batch_solve: load A and b (cvxb_batch_load_eq) first"); return CVXB_E_ARG; }
     CVXB_CUDA(cudaSetDevice(b->device));
     cudaStream_t st = b->st;
     CVXB_TRY(restore_order(b));
     const int n = b->n, m = b->m, T = 256;
+    if (refine > 0 && !b->refw) {
+        // wx x2 (n), wy y2 (p), wz ws z2 s2 t3 (m) per problem
+        const size_t per = 2 * (size_t)n + 2 * (size_t)b->neq + 5 * (size_t)m;
+        cudaError_t e = cudaMalloc(&b->refw, (size_t)b->B * per * sizeof(double));
+        if (e == cudaErrorMemoryAllocation) { cudaGetLastError(); tmp_cache_release(); e = cudaMalloc(&b->refw, (size_t)b->B * per * sizeof(double)); }
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            b->refw = nullptr;
+            set_error("batch_solve: no memory for the refinement workspace");
+            return e == cudaErrorMemoryAllocation ? CVXB_E_NOMEM : CVXB_E_CUDA;
+        }
+        double *w = b->refw;
+        const size_t Bt = b->B;
+        auto take = [&](size_t len) { double *r = w; w += Bt * len; return r; };
+        Ptrs &q = b->p;
+        q.wx = take(n); q.x2 = take(n); q.wy = take(b->neq); q.y2 = take(b->neq);
+        q.wz = take(m); q.ws = take(m); q.z2 = take(m); q.s2 = take(m); q.t3 = take(m);
+    }
     int B = b->B;                                 // active slots: shrinks as problems finish (compaction)
     b->Bact = B;
     Ptrs &p = b->p;
@@ -778,6 +1363,7 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
     b->nsing = 0;
     if (b->neq > 0) CVXB_CUDA(cudaMemsetAsync(p.wsing, 0, (size_t)B * b->neq * sizeof(double), st));
     for (double &t : b->phase_ms) t = 0;
+    for (double &t : b->qphase_ms) t = 0;
     GemvBatch gAt; gAt.batch = B; gAt.sA = b->sA; gAt.sx = b->neq; gAt.sy = n;
     GemvBatch gAn; gAn.batch = B; gAn.sA = b->sA; gAn.sx = n; gAn.sy = b->neq;
     CVXB_CUDA(cudaEventRecord(b->e0, st));
@@ -785,8 +1371,8 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
     k_init_rhs<<<B, T, 0, st>>>(p); count_launch();
     CVXB_TRY(batch_factor(b, true));
     k_scale_bz<<<B, T, 0, st>>>(p, p.dz); count_launch();
-    CVXB_TRY(batch_solve(b));
-    k_init_point<<<B, T, 0, st>>>(p); count_launch();
+    CVXB_TRY(batch_solve(b, p.dx, p.dy));
+    QLAUNCH(k_init_point, B, T, st, p);
     CVXB_LAUNCH_CHECK();
     int info_fail = 0;
     {
@@ -843,14 +1429,33 @@ int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, 
             b->Bact = B;
             gP.batch = gGt.batch = gGn.batch = gAt.batch = gAn.batch = B;
         }
-        k_scaling<<<B, T, 0, st>>>(p, it == 0 ? 1 : 0); count_launch();
+        QLAUNCH(k_scaling, B, T, st, p, it == 0 ? 1 : 0);
         CVXB_TRY(batch_factor(b));
         for (int i = 0; i < 2; ++i) {
-            k_dir_prep<<<B, T, 0, st>>>(p, i); count_launch();
-            CVXB_TRY(batch_solve(b));
-            k_dir_post<<<B, T, 0, st>>>(p, i); count_launch();
+            QLAUNCH(k_dir_prep, B, T, st, p, i, refine > 0 ? 1 : 0);
+            CVXB_TRY(batch_solve(b, p.dx, p.dy));
+            if (refine > 0) {
+                // f4: refine the solution with the residual of the Newton system (:2330-2347)
+                k_f4_post<<<B, T, 0, st>>>(p); count_launch();
+                for (int r = 0; r < refine; ++r) {
+                    QLAUNCH(k_res_prep, B, T, st, p);
+                    CVXB_TRY(gemv_t(n, n, b->P, b->ldp, nullptr, p.dx, -1.0, 1.0, p.x2, st, gP));
+                    if (b->neq > 0) {
+                        CVXB_TRY(gemv_t(b->neq, n, b->A, b->lda, nullptr, p.dy, -1.0, 1.0, p.x2, st, gAt));
+                        CVXB_TRY(gemv_n(b->neq, n, b->A, b->lda, nullptr, p.dx, -1.0, 1.0, p.y2, b->gemv_ws, st, gAn));
+                    }
+                    if (m > 0) {
+                        CVXB_TRY(gemv_t(m, n, b->G, b->ldg, nullptr, p.t3, -1.0, 1.0, p.x2, st, gGt));
+                        CVXB_TRY(gemv_n(m, n, b->G, b->ldg, nullptr, p.dx, -1.0, 1.0, p.z2, b->gemv_ws, st, gGn));
+                    }
+                    QLAUNCH(k_f4_pre, B, T, st, p);
+                    CVXB_TRY(batch_solve(b, p.x2, p.y2));
+                    k_ref_add<<<B, T, 0, st>>>(p); count_launch();
+                }
+            }
+            QLAUNCH(k_dir_post, B, T, st, p, i, refine > 0 ? 1 : 0);
         }
-        k_update<<<B, T, 0, st>>>(p, b->d_info, it); count_launch();
+        QLAUNCH(k_update, B, T, st, p, b->d_info, it);
         CVXB_LAUNCH_CHECK();
     }
     b->iters_run = it;
@@ -925,6 +1530,13 @@ int cvxb_batch_phase_ms(cvxb_batch *b, double *ms) {
     if (!b || !ms) { set_error("batch_phase_ms: NULL argument"); return CVXB_E_ARG; }
     if (!b->time_phases) { set_error("batch_phase_ms: create the batch with CVXB_BATCH_PHASE_MS=1"); return CVXB_E_ARG; }
     for (int k = 0; k < 3; ++k) ms[k] = b->phase_ms[k];
+    return 0;
+}
+
+int cvxb_batch_phase_ms_cones(cvxb_batch *b, double *ms) {
+    if (!b || !ms) { set_error("batch_phase_ms_cones: NULL argument"); return CVXB_E_ARG; }
+    if (!b->time_phases) { set_error("batch_phase_ms_cones: create the batch with CVXB_BATCH_PHASE_MS=1"); return CVXB_E_ARG; }
+    for (int k = 0; k < 2; ++k) ms[k] = b->qphase_ms[k];
     return 0;
 }
 

@@ -208,9 +208,14 @@ int cvxb_gemm(int transa, int transb, int m, int n, int k, double alpha, const d
  * over solvers.qp).  Problems are  min 1/2 x'P x + q'x  s.t.  G x <= h, A x = b,
  * A with p rows (0 <= p <= n; p > 0 needs m > 0).  With p > 0 every problem
  * follows coneqp with kktsolver='chol2' (solvers.qp(P, q, G, h, A, b)).
- * cvxb_batch_create is cvxb_batch_create_eq with p = 0. */
+ * cvxb_batch_create is cvxb_batch_create_eq with p = 0.
+ * cvxb_batch_create_cones: the inequalities are the cone dims = {'l': ml, 'q': [q[0] .. q[nq-1]]}, the same for
+ * every problem: rows of G and h are ml linear rows, then the second-order cones in order (m = ml + sum q, each
+ * q[k] >= 1).  Every problem follows coneqp(P, q, G, h, dims[, A, b]) with the reference's default options.
+ * cvxb_batch_create_eq(.., m, p, ..) is cvxb_batch_create_cones with ml = m, nq = 0. */
 int cvxb_batch_create(cvxb_batch **out, int nprob, int n, int m, int device);
 int cvxb_batch_create_eq(cvxb_batch **out, int nprob, int n, int m, int p, int device);
+int cvxb_batch_create_cones(cvxb_batch **out, int nprob, int n, int ml, int nq, const int *q, int p, int device);
 void cvxb_batch_destroy(cvxb_batch *b);
 /* P: nprob x (n x n, ld n); q: nprob x n; G: nprob x (m x n column-major, ld m); h: nprob x m */
 int cvxb_batch_load(cvxb_batch *b, const double *P, const double *q, const double *G,
@@ -219,6 +224,10 @@ int cvxb_batch_load(cvxb_batch *b, const double *P, const double *q, const doubl
  * cvxb_batch_load when p > 0 (a no-op when p = 0). */
 int cvxb_batch_load_eq(cvxb_batch *b, const double *A, const double *bvec, int space);
 int cvxb_batch_solve(cvxb_batch *b, int maxiters, double abstol, double reltol, double feastol);
+/* the same with coneqp's options['refinement']: steps of iterative refinement per Newton solve; a negative value
+ * is the reference's default (1 with 'q' cones, else 0), which is what cvxb_batch_solve uses */
+int cvxb_batch_solve_ref(cvxb_batch *b, int maxiters, double abstol, double reltol, double feastol,
+                         int refinement);
 /* status: 1 optimal, 2 maximum iterations reached, 3 singular KKT matrix ('unknown' in the
  * reference for 2 and 3).  x/s/z may be device pointers (space), scalars go to host memory. */
 int cvxb_batch_results(cvxb_batch *b, double *x, double *s, double *z, int *status,
@@ -232,6 +241,8 @@ int cvxb_batch_singular(cvxb_batch *b, int *flags);
  * L^{-1} A' (TRSM), A S^{-1} A' (SYRK + Cholesky).  Only for a batch created with
  * CVXB_BATCH_PHASE_MS=1, which synchronises after every phase. */
 int cvxb_batch_phase_ms(cvxb_batch *b, double *ms);
+/* ms[2]: the part of phase S spent on the 'q' rows: Gs_q = W^-T G_q, and the GEMM K += Gs_q' Gs_q (same batches) */
+int cvxb_batch_phase_ms_cones(cvxb_batch *b, double *ms);
 /* CUDA-event time of the last cvxb_batch_solve and the number of lock-step iterations run */
 int cvxb_batch_stats(cvxb_batch *b, double *solve_ms, int *iterations);
 /* kernel of the factorisations' SYRK in the last solve: 1 fp64 DMMA, 2 int8 slices (as cvxb_kkt_syrk_path) */
